@@ -2,6 +2,7 @@
 """bench.py -- full frames/s (voxelize + mip + cone-trace) of the B200 path on BASELINE.json's configs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 1..5] [--mode ...]
+                    [--dump-outputs DIR]
 
 One process per GPU (torchrun for N > 1).  A step is one full frame: sparse clear -> voxelise (coverage + PCF-lit
 shading) -> resolve -> mip pyramid -> primary visibility -> cone trace.  The default workload is config 2 (the one
@@ -90,7 +91,13 @@ def parse(argv=None):
     ap.add_argument("--strong-steps", type=int, default=0, help="timed steps of the config-3 leg (default: min(steps, 40))")
     ap.add_argument("--flush", action="store_true", help="flush L2 between timed steps (per-step events, frames not pipelined); "
                     "default: no flush -- the per-frame working set (~220 MB, two alternating frame slots) exceeds the 126 MB L2")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the frame of the last timed step (config 5: its last probe view) as "
+                         "DIR/frame.npy, float32 RGBA 0..255; a frame over 64 MB is written as DIR/frame_sample.npy, a fixed "
+                         "seeded sample of 2^21 of its pixels.  Inputs are seeded, so two builds can be compared output for output")
     a = ap.parse_args(argv)
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     a.shadow = 4096
     w0, h0 = 1920, 1080
     if a.config == 1:
@@ -419,6 +426,11 @@ def bench_config(env, args):
         env.barrier()
         total_ms = sum(a.elapsed_time(b) for a, b in ev)
     launches = ctx.kernel_launches() - launches0
+    dumped = None
+    if args.dump_outputs and rank == 0:
+        # row-band modes: each rank's own frame holds only its band; the assembled frame is the all-gather's result
+        frame = gather_buf[:H * W * 4].view(H, W, 4).cpu().numpy() if gather_buf is not None else ctx.read_frame()
+        dumped = dump_outputs(frame, args.dump_outputs)
     total_ms = env.max_over_ranks([total_ms])[0]
     frames = args.steps * (world if args.mode == "views" else 64 if args.mode == "probes" else 1)
     value = frames / (total_ms * 1e-3)
@@ -601,7 +613,27 @@ def bench_config(env, args):
         out["cpu_baseline"] = cpu_baseline(args, sc, u, budget_s=15.0)
     if shard_check is not None:
         out["shard_check"] = shard_check
+    if dumped is not None:
+        out["dumped_outputs"] = dumped
     return out
+
+
+DUMP_BYTES = 64_000_000
+DUMP_SAMPLE_PIXELS = 1 << 21
+
+
+def dump_outputs(frame, out_dir):
+    """The frame the last timed step rendered (what vct_frame hands its caller), as float32.  Frames above DUMP_BYTES
+    (config 3: 3840x2160) are sampled: the same pixels, in raster order, on every run of the same frame size."""
+    frame = frame.astype(np.float32)
+    H, W, _ = frame.shape
+    name = "frame"
+    if frame.nbytes > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(0).choice(H * W, size=DUMP_SAMPLE_PIXELS, replace=False))
+        frame, name = frame.reshape(H * W, 4)[idx], "frame_sample"
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), frame)
+    return {name: list(frame.shape)}
 
 
 def voxelize_roofline(ctx, sc, args, passes, fragments, hbm):
