@@ -68,11 +68,8 @@ const char* vct_version(void);
  *           ShardShadowMap (1, set before vct_comm_init: vct_draw_depth rasterises only this rank's triangle share and
  *             min-reduces every depth fragment into all ranks' D24 images -- multimem.red.min.u32 in the NVSwitch; the
  *             resulting map is bit-identical to the single-GPU one.  SURVEY 8e "shadow map")
- *           KeepAccumulator (0: the sparse resolve zeroes the cells it consumes; measured slower, default 1)
  *           ShadowMap VoxelTexture (texture-unit numbers: accepted and ignored)
- *           tuning / diagnostics (defaults are the measured best): DebugConeVariant DebugSpecAhead (cone_trace shapes,
- *             all bit-identical), ChainBlockThreads RasterBlockThreads ConeSmemPad SideStreamsLowPriority PipelineFrames
- *             OverlapVisibility (frame pipeline)
+ *           PipelineFrames OverlapVisibility (frame pipeline; defaults are the measured best)
  *   float : VoxelGridWorldSize ambientFactor DiffuseTanHalfAngle SpecularTanHalfAngle StepMultiplier
  *           MaxDistance MaxAlpha ShadowBias
  *   vec3  : CameraPosition LightDirection

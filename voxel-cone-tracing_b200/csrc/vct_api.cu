@@ -565,14 +565,7 @@ int vct_set_i(vct_handle c, const char* name, int v) {
   else if (k == "SharedRank") { if (v < 0 || v > 15) return set_error(c, VCT_ERR_INVALID, "SharedRank out of range"); c->shared_rank = v; }
   else if (k == "MaxExchangeVoxels") { if (v < 1024) return set_error(c, VCT_ERR_INVALID, "MaxExchangeVoxels too small"); c->exchange_cap_user = (size_t)v; }
   else if (k == "PipelineFrames") c->pipeline_frames = v != 0;
-  else if (k == "DebugSpecAhead") c->debug_spec_ahead = v;
-  else if (k == "DebugConeVariant") c->debug_cone_variant = v;
-  else if (k == "ChainBlockThreads") { if (v != 32 && v != 64 && v != 128 && v != 256) return set_error(c, VCT_ERR_INVALID, "ChainBlockThreads: 32, 64, 128 or 256"); c->chain_block = v; }
-  else if (k == "RasterBlockThreads") { if (v != 32 && v != 64 && v != 128) return set_error(c, VCT_ERR_INVALID, "RasterBlockThreads: 32, 64 or 128"); c->raster_block = v; c->scene_epoch++; }
-  else if (k == "SideStreamsLowPriority") { if (c->stream2) return set_error(c, VCT_ERR_STATE, "SideStreamsLowPriority: set it before the first frame"); c->side_streams_low = v != 0; }
-  else if (k == "ConeSmemPad") { if (v < 0 || v > 40960) return set_error(c, VCT_ERR_INVALID, "ConeSmemPad: 0..40960 bytes"); c->cone_smem_pad = v; }
   else if (k == "DenseResolve") c->dense_resolve = v != 0;
-  else if (k == "KeepAccumulator") { c->keep_accum = v != 0; c->scene_epoch++; }
   else if (k == "ShardShadowMap") { c->shard_shadow = v != 0; c->depth_valid = false; c->scene_epoch++; }
   else if (k == "Profile") {
     c->profile = v != 0;
@@ -601,7 +594,6 @@ int vct_get_i(vct_handle c, const char* name, int* v) {
   else if (k == "RowBegin") *v = P.row_begin; else if (k == "RowEnd") *v = P.row_end;
   else if (k == "RowInterleave") *v = P.row_il; else if (k == "RowPhase") *v = P.row_ph;
   else if (k == "DenseResolve") *v = c->dense_resolve; else if (k == "Profile") *v = c->profile;
-  else if (k == "KeepAccumulator") *v = c->keep_accum;
   else if (k == "ShardShadowMap") *v = c->shard_shadow;
   else return set_error(c, VCT_ERR_INVALID, "unknown int uniform '" + k + "'");
   return VCT_OK;
@@ -948,7 +940,6 @@ static int ensure_overlap(vct_context* c) {
     // scheduler only hands SM slots to another grid ahead of them if that grid's stream has priority
     int prio_lo = 0, prio_hi = 0;
     cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-    if (c->side_streams_low) prio_hi = prio_lo;
     VCT_CUDA(c, cudaStreamCreateWithPriority(&c->stream2, cudaStreamNonBlocking, prio_hi));
     VCT_CUDA(c, cudaEventCreateWithFlags(&c->ev_fork, cudaEventDisableTiming));
     VCT_CUDA(c, cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));

@@ -217,13 +217,12 @@ int launch_visibility(vct_context* c) {
   rc = ensure_vertex_cache(c); if (rc) return rc;
   PassTimer timer(c, VCT_PASS_VISIBILITY);
   const size_t n = (size_t)c->P.W * c->P.H;
-  fill_u64<<<VCT_CHAIN(c, 4), 0, c->stream>>>(c->d_vis2[c->cur], n, ~0ull);
+  fill_u64<<<VCT_CHAIN(4), 0, c->stream>>>(c->d_vis2[c->cur], n, ~0ull);
   VCT_CUDA(c, reset_item_queue(c));
   VisibilityPass pass{c->P, c->vcache2[c->cur], c->d_idx, c->d_trimat, c->d_materials, c->d_vis2[c->cur]};
   const uint32_t nt = (uint32_t)c->nt;
-  raster_small<VisibilityPass><<<(nt + c->raster_block - 1) / c->raster_block, c->raster_block, 0, c->stream>>>(pass, 0, nt, c->d_items,
-                                                                        (uint32_t)c->items_cap, c->d_counters);
-  raster_tiles<VisibilityPass><<<VCT_CHAIN(c, 4), 0, c->stream>>>(pass, c->d_items, (uint32_t)c->items_cap, c->d_counters);
+  raster_small<VisibilityPass><<<(nt + 127) / 128, 128, 0, c->stream>>>(pass, 0, nt, c->d_items, (uint32_t)c->items_cap, c->d_counters);
+  raster_tiles<VisibilityPass><<<VCT_CHAIN(4), 0, c->stream>>>(pass, c->d_items, (uint32_t)c->items_cap, c->d_counters);
   c->launches += 3;
   VCT_CUDA(c, cudaGetLastError());
   return VCT_OK;
@@ -397,7 +396,8 @@ __device__ __forceinline__ unsigned char to_unorm8(float x) {
 
 // one warp = 8x4 pixels; block = 2 warps = 8x8 pixels (small blocks: the specular chain length varies a lot
 // between warps and a block holds its registers until its slowest warp is done)
-template <int NC, int SU, int BT, int MINB>
+constexpr int BT = 64;
+template <int NC, int SU, int MINB>
 __global__ void __launch_bounds__(BT, MINB) cone_trace(Params P, VertexCache vc,
                                                   const uint32_t* __restrict__ idx,
                                                   const uint16_t* __restrict__ trimat,
@@ -411,8 +411,8 @@ __global__ void __launch_bounds__(BT, MINB) cone_trace(Params P, VertexCache vc,
   const int lx = lane & 7, ly = lane >> 3;    // 8x4 pixel tile per warp (a 2x2-quad lane order measured the same)
   const int i = blockIdx.x * 8 + lx;
   // rows of this block: contiguous from y_begin, or (interleaved strips) the blockIdx.y-th owned group of 8 rows
-  const int j = P.row_il > 1 ? (((int)blockIdx.y / (64 / BT)) * P.row_il + P.row_ph) * 8 + ((int)blockIdx.y % (64 / BT)) * (BT / 8) + warp * 4 + ly
-                             : y_begin + (int)blockIdx.y * (BT / 8) + warp * 4 + ly;
+  const int j = P.row_il > 1 ? ((int)blockIdx.y * P.row_il + P.row_ph) * 8 + warp * 4 + ly
+                             : y_begin + (int)blockIdx.y * 8 + warp * 4 + ly;
   unsigned samples = 0;
   if (i < P.W && j < y_end) {
     const unsigned long long key = vis[(size_t)j * P.W + i];
@@ -552,42 +552,17 @@ int launch_cone(vct_context* c) {
     if (!own_groups) return VCT_OK;
   }
   if (y0 >= y1) return VCT_OK;
-  // NC = 6 (the reference's table) has tuning variants selected by DebugConeVariant: specular fetch-ahead depth SU,
-  // block size BT (one or two 8x4 warp tiles), register budget via MINB blocks per SM.  All variants execute the same
-  // arithmetic per pixel: frames are bit-identical (test_cone_trace_variants_are_bit_identical).
-#define VCT_LAUNCH_CONE(NC, SU, BT, MINB)                                                                              \
+  // one shape per cone table: specular fetch-ahead depth SU and register budget via MINB blocks per SM, the fastest
+  // measured; <9, 2, 64, 8> and <9, 2, 32, 16> are miscompiled by nvcc 12.9 (profiles/r02_cone_variants.txt)
+#define VCT_LAUNCH_CONE(NC, SU, MINB)                                                                                  \
   do {                                                                                                                 \
-    dim3 b(BT), g((c->P.W + 7) / 8, strips ? own_groups * (64 / BT) : (y1 - y0 + (BT / 8) - 1) / (BT / 8));            \
-    cone_trace<NC, SU, BT, MINB><<<g, b, 3 * NC * BT * sizeof(float) + (size_t)c->cone_smem_pad, c->stream>>>(c->P, c->vcache2[c->cur], c->d_idx,  \
+    dim3 b(BT), g((c->P.W + 7) / 8, strips ? own_groups : (y1 - y0 + 7) / 8);                                          \
+    cone_trace<NC, SU, MINB><<<g, b, 3 * NC * BT * sizeof(float), c->stream>>>(c->P, c->vcache2[c->cur], c->d_idx,     \
         c->d_trimat, c->d_materials, c->d_depth, c->d_vis2[c->cur], c->grid[c->cur].tex, c->d_frame, c->d_counters, y0, y1); \
   } while (0)
-  const int su = c->debug_spec_ahead;
-  if (c->P.n_cones <= 6) {
-    switch (strips && c->debug_cone_variant == 8 ? 0 : c->debug_cone_variant) {   // (128-thread blocks span two strips)
-      case 1: VCT_LAUNCH_CONE(6, 4, 64, 8); break;        // round-1 shape: 128 registers, 8 blocks / SM
-      case 2: VCT_LAUNCH_CONE(6, 2, 64, 10); break;
-      case 3: VCT_LAUNCH_CONE(6, 4, 32, 16); break;
-      case 4: VCT_LAUNCH_CONE(6, 4, 32, 20); break;
-      case 5: VCT_LAUNCH_CONE(6, 2, 32, 20); break;
-      case 8: VCT_LAUNCH_CONE(6, 4, 128, 4); break;
-      default:                                            // 96 registers, 10 blocks / SM: +2.4 % on config 2 (profiles/r02_cone_variants.txt)
-        if (su == 1) VCT_LAUNCH_CONE(6, 1, 64, 8); else if (su == 2) VCT_LAUNCH_CONE(6, 2, 64, 8); else VCT_LAUNCH_CONE(6, 4, 64, 10);
-    }
-  } else if (c->P.n_cones <= 9) {                         // BASELINE config 3: 9 diffuse cones + specular
-    switch (c->debug_cone_variant) {
-      case 1: VCT_LAUNCH_CONE(16, 2, 64, 8); break;       // round-1 shape (16-cone template)
-      case 3: VCT_LAUNCH_CONE(9, 2, 64, 10); break;
-      case 4: VCT_LAUNCH_CONE(9, 4, 32, 16); break;
-      // NOT offered: <9, 2, 64, 8> and <9, 2, 32, 16>.  nvcc 12.9.86 generates code for these two instantiations (128
-      // registers, no spills) that drops ~0.4 % of the march steps -- same source, same inputs; <9, 2, 64, 10>, <9, 4, ..>,
-      // <9, 1, ..> and <16, 2, ..> agree with each other and with the oracle (tools/variant_diff.py,
-      // profiles/r02_cone_variants.txt).  test_cone_trace_variants_are_bit_identical pins every variant that IS offered.
-      default:                                            // 9-cone template + 4 specular steps ahead: -10 % vs the 16-cone template
-        if (su == 1) VCT_LAUNCH_CONE(9, 1, 64, 8); else if (su == 2) VCT_LAUNCH_CONE(9, 2, 64, 10); else VCT_LAUNCH_CONE(9, 4, 64, 8);
-    }
-  } else {
-    if (su == 1) VCT_LAUNCH_CONE(16, 1, 64, 8); else VCT_LAUNCH_CONE(16, 2, 64, 8);
-  }
+  if (c->P.n_cones <= 6) VCT_LAUNCH_CONE(6, 4, 10);       // 96 registers, 10 blocks / SM: +2.4 % on config 2
+  else if (c->P.n_cones <= 9) VCT_LAUNCH_CONE(9, 4, 8);   // BASELINE config 3: -10 % vs the 16-cone template
+  else VCT_LAUNCH_CONE(16, 2, 8);
 #undef VCT_LAUNCH_CONE
   c->launches += 1;
   c->last_frame = c->d_frame;

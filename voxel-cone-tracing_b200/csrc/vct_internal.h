@@ -98,17 +98,7 @@ struct vct_context {
   int dense_resolve = 0;
   int shard_shadow = 0;         // 1 (set before vct_comm_init): vct_draw_depth rasterises this rank's triangle share and
                                 // min-reduces it into every rank's D24 image through the switch (multimem.red.min.u32)
-  int keep_accum = 1;           // 0: the sparse resolve zeroes every accumulator cell it consumes (no separate clear of the
-                                // accumulator next frame); vct_readback_counts / _sums then have nothing to read
   int grid_format = 0;
-  int debug_spec_ahead = 4;   // specular steps fetched ahead per iteration (1, 2, 4)
-  int debug_cone_variant = 0; // cone_trace tuning variant (block size / register budget / fetch-ahead), see launch_cone
-  // Overlap tuning (frames pipeline: the voxel chain of frame i+1 runs beside cone_trace of frame i, which fills the
-  // register file with its own blocks).  chain_block: threads per block of the grid-stride kernels of the voxel chain
-  // (small blocks slot into the registers a retiring cone_trace block frees); raster_block: the same for raster_small;
-  // cone_smem_pad: extra dynamic shared memory per cone_trace block, i.e. a cap on its blocks per SM that leaves room.
-  int chain_block = 256, raster_block = 128, cone_smem_pad = 0;
-  int side_streams_low = 0;   // 1: the voxel / visibility streams get the LOWEST priority (set before the first frame)
   size_t max_fragments = 16u << 20;
   size_t max_items = 4u << 20;
 
@@ -258,8 +248,8 @@ int comm_check(vct_context* c);                                        // barrie
 bool comm_depth_views(vct_context* c, uint32_t** local, uint32_t** mc, uint32_t** peers, size_t* seg_words, int* world, int* rank);
 void comm_release_for_destroy(vct_context* c);
 int sync_all_streams(vct_context* c);      // main + voxel + visibility + copy streams idle (before freeing what frames in flight read)
-// launch shape of a grid-stride kernel of the voxel chain: `mult` x 256 threads per SM in blocks of chain_block threads
-#define VCT_CHAIN(c, mult) (unsigned)(148 * (mult) * 256 / (c)->chain_block), (unsigned)(c)->chain_block
+// launch shape of a grid-stride kernel of the voxel chain: `mult` blocks of 256 threads per SM
+#define VCT_CHAIN(mult) (unsigned)(148 * (mult)), 256u
 inline cudaError_t reset_item_queue(vct_context* c) { return cudaMemsetAsync(&c->d_counters->n_items, 0, 3 * sizeof(unsigned int), c->stream); }
 
 // ------------------------------------------------------------------------------------ device helpers

@@ -428,9 +428,9 @@ __device__ __forceinline__ uint2 resolve_cell16(unsigned long long rg, unsigned 
 // per voxel: every thread keeps ILP of them in flight (list entries first, then the cells, then the work).
 constexpr int ILP = 4;
 
-__global__ void vox_resolve_sparse(unsigned long long* __restrict__ accum,
+__global__ void vox_resolve_sparse(const unsigned long long* __restrict__ accum,
                                    const uint32_t* __restrict__ touched, const unsigned int* __restrict__ n_touched,
-                                   cudaSurfaceObject_t level0, int V, int f16, unsigned char* __restrict__ dirty, int zero_after) {
+                                   cudaSurfaceObject_t level0, int V, int f16, unsigned char* __restrict__ dirty) {
   const uint32_t n = *n_touched;
   const uint32_t stride = gridDim.x * blockDim.x;
   for (uint32_t k0 = blockIdx.x * blockDim.x + threadIdx.x; k0 < n; k0 += ILP * stride) {
@@ -444,8 +444,6 @@ __global__ void vox_resolve_sparse(unsigned long long* __restrict__ accum,
 #pragma unroll
     for (int m = 0; m < ILP; ++m) {
       if (v[m] == 0xFFFFFFFFu) continue;
-      // KeepAccumulator = 0: the cell is consumed here and zeroed while its sector is at hand
-      if (zero_after) *reinterpret_cast<ulonglong2*>(&accum[2 * (size_t)v[m]]) = make_ulonglong2(0ull, 0ull);
       int x = v[m] % V, y = (v[m] / V) % V, z = v[m] / (V * V);
       if (f16) surf3Dwrite(resolve_cell16(a[m].x, a[m].y), level0, x * 8, y, z);
       else surf3Dwrite(resolve_cell(a[m].x, a[m].y), level0, x * 4, y, z);
@@ -479,8 +477,8 @@ int launch_voxel_clear(vct_context* c) {
   PassTimer timer(c, VCT_PASS_VOX_CLEAR);
   const int V = c->P.V;
   vct_context::GridBuf& g = c->grid[c->cur];
-  // accumulator: all zero already (the last sparse resolve zeroed what it consumed, KeepAccumulator = 0), or described by
-  // a slot's touched list (sparse clear), or unknown (dense memset)
+  // accumulator: all zero already (vox_push_shared left it so), or described by a slot's touched list (sparse clear), or
+  // unknown (dense memset)
   const bool accum_clean = c->accum_list_slot == -2 && !c->dense_resolve;
   const bool accum_sparse = c->accum_list_slot >= 0 && !c->dense_resolve;
   if (!accum_sparse && !accum_clean) VCT_CUDA(c, cudaMemsetAsync(c->d_accum, 0, (size_t)V * V * V * 16, c->stream));
@@ -503,8 +501,8 @@ int launch_voxel_clear(vct_context* c) {
   }
   if (accum_sparse || g.list_valid) {
     const vct_context::GridBuf* a = accum_sparse ? &c->grid[c->accum_list_slot] : nullptr;
-    vox_clear_sparse<<<VCT_CHAIN(c, 8), 0, c->stream>>>(c->d_accum, a ? a->touched : nullptr, a ? a->n_touched : nullptr,
-                                                     g.surf[0], g.list_valid ? g.touched : nullptr, g.n_touched, V, c->grid_format);
+    vox_clear_sparse<<<VCT_CHAIN(8), 0, c->stream>>>(c->d_accum, a ? a->touched : nullptr, a ? a->n_touched : nullptr,
+                                                  g.surf[0], g.list_valid ? g.touched : nullptr, g.n_touched, V, c->grid_format);
     c->launches += 1;
   }
   VCT_CUDA(c, cudaMemsetAsync(g.n_touched, 0, sizeof(unsigned int), c->stream));
@@ -536,24 +534,23 @@ static int voxelize_impl(vct_context* c, size_t tb, size_t te, int shared) {
     VCT_CUDA(c, cudaMemsetAsync(&c->d_counters->n_fragments, 0, sizeof(unsigned int), c->stream));
     VoxCoverPass pass{c->P, c->vcache2[c->cur], c->d_idx, c->d_trimat, c->d_materials, (VoxRecord*)c->d_voxrec, c->d_frags, (uint32_t)c->frags_cap, c->d_counters};
     const uint32_t n = (uint32_t)(te - tb);
-    const uint32_t rb = (uint32_t)c->raster_block;
-    const uint32_t n_blocks = (n + rb - 1) / rb, il = (uint32_t)c->tri_interleave, ph = (uint32_t)c->tri_phase % il;
+    const uint32_t n_blocks = (n + 127) / 128, il = (uint32_t)c->tri_interleave, ph = (uint32_t)c->tri_phase % il;
     const uint32_t own_blocks = n_blocks > ph ? (n_blocks - ph + il - 1) / il : 0;
     if (own_blocks)
-      raster_small<VoxCoverPass><<<own_blocks, rb, 0, c->stream>>>(pass, (uint32_t)tb, (uint32_t)te, c->d_items,
-                                                                    (uint32_t)c->items_cap, c->d_counters, il, ph);
-    raster_tiles<VoxCoverPass><<<VCT_CHAIN(c, 4), 0, c->stream>>>(pass, c->d_items, (uint32_t)c->items_cap, c->d_counters);
+      raster_small<VoxCoverPass><<<own_blocks, 128, 0, c->stream>>>(pass, (uint32_t)tb, (uint32_t)te, c->d_items,
+                                                                     (uint32_t)c->items_cap, c->d_counters, il, ph);
+    raster_tiles<VoxCoverPass><<<VCT_CHAIN(4), 0, c->stream>>>(pass, c->d_items, (uint32_t)c->items_cap, c->d_counters);
     c->launches += 2;
   }
   {
     PassTimer timer(c, VCT_PASS_VOX_SHADE);
     uint32_t* list = shared ? c->d_push_list : c->grid[c->cur].touched;
     unsigned int* n_list = shared ? c->d_push_count : c->grid[c->cur].n_touched;
-    vox_shade<<<VCT_CHAIN(c, 8), 0, c->stream>>>(c->P, (const VoxRecord*)c->d_voxrec, c->d_materials, c->d_depth,
-                                              c->depth_tex, c->d_frags, (uint32_t)c->frags_cap, c->d_accum, c->d_occ_mask,
-                                              c->d_counters);
+    vox_shade<<<VCT_CHAIN(8), 0, c->stream>>>(c->P, (const VoxRecord*)c->d_voxrec, c->d_materials, c->d_depth,
+                                           c->depth_tex, c->d_frags, (uint32_t)c->frags_cap, c->d_accum, c->d_occ_mask,
+                                           c->d_counters);
     const uint32_t n_words = (uint32_t)(((size_t)c->P.V * c->P.V * c->P.V + 31) / 32);
-    vox_compact_mask<<<VCT_CHAIN(c, 4), 0, c->stream>>>(c->d_occ_mask, n_words, list, n_list);
+    vox_compact_mask<<<VCT_CHAIN(4), 0, c->stream>>>(c->d_occ_mask, n_words, list, n_list);
     c->launches += 2;
   }
   VCT_CUDA(c, cudaGetLastError());
@@ -711,9 +708,9 @@ int launch_voxelize_shared(vct_context* c, size_t tb, size_t te) {
   {
     PassTimer timer(c, VCT_PASS_EXCHANGE_PUSH);
     if (c->shared_mc)
-      vox_push_shared<true><<<VCT_CHAIN(c, 8), 0, c->stream>>>(c->d_accum, c->d_push_list, c->d_push_count, (float4*)c->shared_mc, c->P.V);
+      vox_push_shared<true><<<VCT_CHAIN(8), 0, c->stream>>>(c->d_accum, c->d_push_list, c->d_push_count, (float4*)c->shared_mc, c->P.V);
     else
-      vox_push_shared<false><<<VCT_CHAIN(c, 8), 0, c->stream>>>(c->d_accum, c->d_push_list, c->d_push_count, (float4*)c->shared_local, c->P.V);
+      vox_push_shared<false><<<VCT_CHAIN(8), 0, c->stream>>>(c->d_accum, c->d_push_list, c->d_push_count, (float4*)c->shared_local, c->P.V);
     c->launches += 1;
   }
   VCT_CUDA(c, cudaGetLastError());
@@ -782,7 +779,7 @@ int launch_resolve_shared(vct_context* c) {
     c->launches += 1;
   }
   uint32_t* mask = reinterpret_cast<uint32_t*>(c->shared_local + 2 * (size_t)V * V * V);
-  vox_resolve_shared<<<VCT_CHAIN(c, 8), 0, c->stream>>>(c->shared_local, mask, c->mask_prev[c->cur], g.surf[0], V, c->grid_format);
+  vox_resolve_shared<<<VCT_CHAIN(8), 0, c->stream>>>(c->shared_local, mask, c->mask_prev[c->cur], g.surf[0], V, c->grid_format);
   c->launches += 1;
   // the slot is now described by mask_prev, not by a touched list: a later private-accumulator voxelisation into
   // this slot must start from a dense zero, and mask_prev stays exact as long as only this path writes the slot
@@ -805,14 +802,14 @@ static int voxelize_inbox(vct_context* c, size_t tb, size_t te, bool slot_ready)
   const uint32_t cap = (uint32_t)c->exchange_cap;
   PassTimer timer(c, VCT_PASS_EXCHANGE_PUSH);
   if (c->shared_mc)
-    vox_push_inbox<1><<<VCT_CHAIN(c, 4), 0, c->stream>>>(c->d_accum, g.touched, g.n_touched, (unsigned char*)c->shared_mc, 0,
-                                                      c->exchange_parity, c->shared_world, c->shared_rank, cap, c->d_counters);
+    vox_push_inbox<1><<<VCT_CHAIN(4), 0, c->stream>>>(c->d_accum, g.touched, g.n_touched, (unsigned char*)c->shared_mc, 0,
+                                                   c->exchange_parity, c->shared_world, c->shared_rank, cap, c->d_counters);
   else if (c->shared_peers && c->shared_world > 1)
-    vox_push_inbox<2><<<VCT_CHAIN(c, 4), 0, c->stream>>>(c->d_accum, g.touched, g.n_touched, c->shared_peers, c->shared_seg,
-                                                      c->exchange_parity, c->shared_world, c->shared_rank, cap, c->d_counters);
+    vox_push_inbox<2><<<VCT_CHAIN(4), 0, c->stream>>>(c->d_accum, g.touched, g.n_touched, c->shared_peers, c->shared_seg,
+                                                   c->exchange_parity, c->shared_world, c->shared_rank, cap, c->d_counters);
   else
-    vox_push_inbox<0><<<VCT_CHAIN(c, 4), 0, c->stream>>>(c->d_accum, g.touched, g.n_touched, (unsigned char*)c->shared_local, 0,
-                                                      c->exchange_parity, c->shared_world, c->shared_rank, cap, c->d_counters);
+    vox_push_inbox<0><<<VCT_CHAIN(4), 0, c->stream>>>(c->d_accum, g.touched, g.n_touched, (unsigned char*)c->shared_local, 0,
+                                                   c->exchange_parity, c->shared_world, c->shared_rank, cap, c->d_counters);
   // own record count, needed by the merge for the overflow check (the list keeps growing during the merge)
   if (!c->d_push_count) VCT_CUDA(c, cudaMalloc(&c->d_push_count, 128));
   VCT_CUDA(c, cudaMemcpyAsync(c->d_push_count, g.n_touched, 4, cudaMemcpyDeviceToDevice, c->stream));
@@ -829,9 +826,9 @@ static int resolve_inbox(vct_context* c) {
     // read-modify-write.  (All ranks in one launch with atomic adds was measured: 185 us instead of 89 at four ranks.)
     for (int r = 0; r < c->shared_world; ++r) {
       if (r == c->shared_rank) continue;
-      vox_merge_inbox<<<VCT_CHAIN(c, 4), 0, c->stream>>>(c->d_accum, (const unsigned char*)c->shared_local, c->exchange_parity,
-                                                      c->shared_world, r, (uint32_t)c->exchange_cap, g.touched, g.n_touched,
-                                                      c->d_counters, c->d_push_count);
+      vox_merge_inbox<<<VCT_CHAIN(4), 0, c->stream>>>(c->d_accum, (const unsigned char*)c->shared_local, c->exchange_parity,
+                                                   c->shared_world, r, (uint32_t)c->exchange_cap, g.touched, g.n_touched,
+                                                   c->d_counters, c->d_push_count);
       c->launches += 1;
     }
   }
@@ -854,10 +851,8 @@ int launch_resolve(vct_context* c, bool dense) {
     c->mask_valid[c->cur] = false;
     c->accum_list_slot = -1;
   } else {
-    const int zero_after = c->keep_accum ? 0 : 1;
-    vox_resolve_sparse<<<VCT_CHAIN(c, 8), 0, c->stream>>>(c->d_accum, g.touched, g.n_touched, g.surf[0], V, c->grid_format, g.dirty_now, zero_after);
+    vox_resolve_sparse<<<VCT_CHAIN(8), 0, c->stream>>>(c->d_accum, g.touched, g.n_touched, g.surf[0], V, c->grid_format, g.dirty_now);
     g.occ_valid = g.list_valid;
-    if (zero_after && c->accum_list_slot == c->cur) c->accum_list_slot = -2;     // every non-zero cell was on this list
   }
   g.mips_current = false;
   c->launches += 1;
@@ -867,7 +862,6 @@ int launch_resolve(vct_context* c, bool dense) {
 
 int readback_accum(vct_context* c, uint32_t* counts, uint32_t* sums) {
   int rc = ensure_grid(c); if (rc) return rc;
-  if (!c->keep_accum) return set_error(c, VCT_ERR_STATE, "the accumulator is consumed by the resolve (KeepAccumulator = 0): nothing to read back");
   const size_t n = (size_t)c->P.V * c->P.V * c->P.V;
   uint32_t *dc = nullptr, *ds = nullptr;
   if (counts) VCT_CUDA(c, cudaMalloc(&dc, n * 4));
