@@ -44,7 +44,8 @@ typedef enum vct_pass {
   VCT_PASS_REINJECT = 9,    /* Bounces >= 3 extension                                               */
   VCT_PASS_EXCHANGE_PUSH = 10,  /* vct_voxelize_shared: multicast of the touched voxels (multimem.st / multimem.red) */
   VCT_PASS_EXCHANGE_MERGE = 11, /* vct_resolve_shared (inbox): the other ranks' records added to the accumulator     */
-  VCT_PASS_COUNT = 12
+  VCT_PASS_VOXEL_VIEW = 12, /* vct_render_voxels (no reference counterpart)                          */
+  VCT_PASS_COUNT = 13
 } vct_pass;
 
 /* ---- lifetime.  Replaces Voxel_Cone_Tracing::Voxel_Cone_Tracing + init_voxel_cone_tracing resource
@@ -106,6 +107,15 @@ int vct_draw_voxels(vct_handle h);       /* DrawVoxelTexture   Voxel_Cone_Tracin
 int vct_render(vct_handle h, uint8_t* host_rgba);
 /* vct_draw_voxels + vct_render as one call (what the metric "full frames/s" times) */
 int vct_frame(vct_handle h, uint8_t* host_rgba);
+/* Voxel view (no reference counterpart): the W*H view of mip level `level` of the current pyramid from the camera of
+ * vct_render (ModelMatrix, ModelViewMatrix, ProjectionMatrix, screen size).  Each pixel shows the first occupied texel
+ * its ray meets between the near and far planes, un-premultiplied and shaded by the axis of the face it entered through;
+ * a miss shows the frame background.  host_rgba (H*W*4, row 0 = bottom row) and host_voxel (H*W texel indices
+ * (z*N+y)*N+x at that level, 0xFFFFFFFF = miss) may each be NULL; with both NULL the call is asynchronous.  Writes the
+ * frame buffer (vct_readback_frame / vct_frame_buffer return the view), renders every row whatever the row-sharding
+ * uniforms say, and is stream-ordered after earlier frames.  VCT_ERR_INVALID: level outside [0, levels);
+ * VCT_ERR_STATE: level > 0 after vct_upload_grid_level0 without vct_build_mips.  DESIGN.md section 3 "Voxel view". */
+int vct_render_voxels(vct_handle h, int level, uint8_t* host_rgba, uint32_t* host_voxel);
 
 /* Pipelined form of vct_frame for render loops (the reference's loop is glClear -> Render -> glfwSwapBuffers,
  * main.cpp:77-94; swapping is what lets a GL driver overlap frames).  vct_frame_async renders into one of a ring
@@ -207,7 +217,8 @@ int vct_frame_buffer(vct_handle h, void** device_ptr, size_t* n_bytes);
 int vct_cone_samples(vct_handle h, uint64_t* n);       /* textureLod calls of the last vct_render */
 int vct_fragment_count(vct_handle h, uint64_t* n);     /* fragments of the last voxelisation */
 int vct_occupied_voxels(vct_handle h, uint64_t* n);
-int vct_debug_counter(vct_handle h, int which, uint64_t* n);   /* diagnostics: 0 = tile work items of the last raster pass */
+/* diagnostics: 0 = tile work items of the last raster pass, 1 = texels the last voxel view visited (all pixels) */
+int vct_debug_counter(vct_handle h, int which, uint64_t* n);
 
 /* ---- cone queries: Voxel_Cone_Tracing(direction, tanHalfAngle) (VoxelConeTracing.fs:82-107) for arbitrary
  * start points (already offset along the normal, :92).  Host arrays: starts/dirs n*3, tan_half n,

@@ -4,6 +4,7 @@ events (main.cpp:77-150), one PNG / PPM per frame instead of glfwSwapBuffers.
 
     python tools/flythrough.py --scene atrium --grid 256 --size 1280x720 --script "W*30 D*10 M(120,0) W*20 S(-10)" --out fly_%04d.png
     python tools/flythrough.py --script "W*3 M(90,0) E*2" --dry-run        # camera path only, no device needed
+    python tools/flythrough.py --scene atrium --grid 256 --voxels 2 --out vox_%04d.png   # mip level 2 as cubes instead
 
 Script tokens (each yields one frame; `*n` repeats): W S A D = forward / back / left / right as main.cpp:136-143 binds
 them, E Q = the enum's UP / DOWN (Camera.h:16-17; the reference binds no key to them) -- ProcessKeyBoard with
@@ -59,6 +60,8 @@ def main(argv=None):
     ap.add_argument("--dt", type=float, default=1.0 / 60.0 * 20, help="deltaTime handed to ProcessKeyBoard per frame (seconds)")
     ap.add_argument("--out", default="fly_%04d.png", help="printf pattern; .png or .ppm")
     ap.add_argument("--dry-run", action="store_true", help="print the camera path and exit (no CUDA device needed)")
+    ap.add_argument("--voxels", type=int, default=None, metavar="LEVEL",
+                    help="write voxel views of mip LEVEL (the grid drawn as cubes, vct_render_voxels) instead of frames")
     a = ap.parse_args(argv)
     w, h = (int(x) for x in a.size.lower().split("x"))
     sc = {"cornell": scenes.cornell, "atrium": scenes.atrium, "knot": scenes.dynamic_knot}[a.scene]()
@@ -74,11 +77,14 @@ def main(argv=None):
     frame = np.empty((h, w, 4), dtype=np.uint8)
     for k, ev in enumerate(events):
         apply(cam, ev, a.dt)
-        r.Render(frame)                                # reads camera.GetViewMatrix() / Zoom, as Render() does (:161-165)
+        if a.voxels is None:
+            r.Render(frame)                            # reads camera.GetViewMatrix() / Zoom, as Render() does (:161-165)
+        else:
+            r.RenderVoxels(a.voxels, frame)            # same camera, the pyramid's level instead of the shaded frame
         path = a.out % k
         top_down = np.ascontiguousarray(frame[::-1, :, :3])    # GL rows run bottom-up
         (images.save_pnm if path.endswith((".ppm", ".pgm")) else images.save_png)(top_down, path)
-    print(f"{len(events)} frames -> {a.out}")
+    print(f"{len(events)} {'frames' if a.voxels is None else f'voxel views of level {a.voxels}'} -> {a.out}")
     return cam
 
 

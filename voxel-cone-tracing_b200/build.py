@@ -16,7 +16,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libvct_b200.so")
-SOURCES = ["vct_api.cu", "vct_shadow.cu", "vct_voxelize.cu", "vct_mip.cu", "vct_cone.cu", "vct_comm.cu"]
+SOURCES = ["vct_api.cu", "vct_shadow.cu", "vct_voxelize.cu", "vct_mip.cu", "vct_cone.cu", "vct_comm.cu", "vct_view.cu"]
 HEADERS = ["vct_internal.h", "vct_raster.cuh", os.path.join("..", "..", "include", "vct_c_api.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "--fmad=false", "-std=c++17",
               "-Xcompiler", "-fPIC,-O2", "--expt-relaxed-constexpr", "-cudart", "static"]

@@ -11,13 +11,15 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libvct_b200.so")
 
 PASSES = {"depth": 0, "vox_clear": 1, "vox_cover": 2, "vox_shade": 3, "resolve": 4, "mip": 5,
-          "visibility": 6, "cone": 7, "frame": 8, "reinject": 9, "exchange_push": 10, "exchange_merge": 11}
+          "visibility": 6, "cone": 7, "frame": 8, "reinject": 9, "exchange_push": 10, "exchange_merge": 11,
+          "voxel_view": 12}
 
 # every symbol include/vct_c_api.h declares (tests check the library exports all of them)
 SYMBOLS = [
     "vct_create", "vct_destroy", "vct_last_error", "vct_version", "vct_set_i", "vct_set_f", "vct_set_3f",
     "vct_set_mat4", "vct_get_i", "vct_get_f", "vct_set_cones", "vct_upload_texture", "vct_set_material",
     "vct_upload_mesh", "vct_update_positions", "vct_draw_depth", "vct_draw_voxels", "vct_render", "vct_frame", "vct_frame_async", "vct_frame_wait",
+    "vct_render_voxels",
     "vct_voxelize_range", "vct_accum_buffer", "vct_resolve_and_mip", "vct_shared_accum_bytes", "vct_set_shared_accum",
     "vct_voxelize_shared", "vct_resolve_shared", "vct_frame_shared_begin", "vct_exchange_stream", "vct_frame_shared_end", "vct_readback_depth", "vct_readback_counts",
     "vct_readback_sums", "vct_readback_grid", "vct_upload_grid_level0", "vct_build_mips", "vct_readback_visibility",
@@ -61,7 +63,7 @@ def load_library(path=None):
         "vct_set_cones": [vp, i, vp, vp], "vct_upload_texture": [vp, i, i, i, i, vp],
         "vct_set_material": [vp, i, i, i, i, f], "vct_upload_mesh": [vp, vp, sz, vp, sz, vp],
         "vct_update_positions": [vp, vp, sz, i], "vct_draw_depth": [vp], "vct_draw_voxels": [vp],
-        "vct_render": [vp, vp], "vct_frame": [vp, vp], "vct_frame_async": [vp, vp], "vct_frame_wait": [vp], "vct_voxelize_range": [vp, sz, sz, i],
+        "vct_render": [vp, vp], "vct_render_voxels": [vp, i, vp, vp], "vct_frame": [vp, vp], "vct_frame_async": [vp, vp], "vct_frame_wait": [vp], "vct_voxelize_range": [vp, sz, sz, i],
         "vct_accum_buffer": [vp, C.POINTER(vp), C.POINTER(sz)], "vct_resolve_and_mip": [vp],
         "vct_shared_accum_bytes": [vp, C.POINTER(sz)], "vct_set_shared_accum": [vp, vp, vp],
         "vct_voxelize_shared": [vp, sz, sz], "vct_resolve_shared": [vp],
@@ -224,6 +226,13 @@ class Context:
 
     def frame(self, out=None):
         self._ck(self.L.vct_frame(self.h, None if out is None else _host_ptr(out)))
+
+    def render_voxels(self, level, out=None, voxel=None):
+        """Voxel view of mip `level` from the render camera into the frame buffer.  `out`: optional host buffer for the
+        (H, W, 4) uint8 view, `voxel`: optional host buffer for the (H, W) uint32 texel indices (0xFFFFFFFF = miss);
+        with neither the call stays on the device and is asynchronous."""
+        self._ck(self.L.vct_render_voxels(self.h, int(level), None if out is None else _host_ptr(out),
+                                          None if voxel is None else _host_ptr(voxel)))
 
     def frame_async(self, out):
         """Pipelined frame: renders and queues the copy into `out` (pinned host buffer); see frame_wait()."""

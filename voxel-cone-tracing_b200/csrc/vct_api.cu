@@ -934,6 +934,78 @@ int vct_render(vct_handle c, uint8_t* host_rgba) {
   return VCT_OK;
 }
 
+// ---- voxel view
+// C = A * B for column-major 4x4 matrices, double, glm's operator* order: column j = ((A0 b0j + A1 b1j) + A2 b2j) + A3 b3j
+static void mat4_mul(const double* A, const double* B, double* C) {
+  for (int j = 0; j < 4; ++j)
+    for (int i = 0; i < 4; ++i)
+      C[j * 4 + i] = ((A[0 * 4 + i] * B[j * 4 + 0] + A[1 * 4 + i] * B[j * 4 + 1]) + A[2 * 4 + i] * B[j * 4 + 2]) +
+                     A[3 * 4 + i] * B[j * 4 + 3];
+}
+
+// glm::inverse(mat4) (glm/detail/func_matrix.inl, compute_inverse<4, 4>): cofactors, then times 1 / determinant.
+// m[c][r] = column c, row r.  The CPU reference of the tests writes out the same operations in the same order (DESIGN.md section 3).
+static void mat4_inverse_glm(const double* a, double* out) {
+  auto m = [&](int c, int r) { return a[c * 4 + r]; };
+  const double c00 = m(2, 2) * m(3, 3) - m(3, 2) * m(2, 3), c02 = m(1, 2) * m(3, 3) - m(3, 2) * m(1, 3), c03 = m(1, 2) * m(2, 3) - m(2, 2) * m(1, 3);
+  const double c04 = m(2, 1) * m(3, 3) - m(3, 1) * m(2, 3), c06 = m(1, 1) * m(3, 3) - m(3, 1) * m(1, 3), c07 = m(1, 1) * m(2, 3) - m(2, 1) * m(1, 3);
+  const double c08 = m(2, 1) * m(3, 2) - m(3, 1) * m(2, 2), c10 = m(1, 1) * m(3, 2) - m(3, 1) * m(1, 2), c11 = m(1, 1) * m(2, 2) - m(2, 1) * m(1, 2);
+  const double c12 = m(2, 0) * m(3, 3) - m(3, 0) * m(2, 3), c14 = m(1, 0) * m(3, 3) - m(3, 0) * m(1, 3), c15 = m(1, 0) * m(2, 3) - m(2, 0) * m(1, 3);
+  const double c16 = m(2, 0) * m(3, 2) - m(3, 0) * m(2, 2), c18 = m(1, 0) * m(3, 2) - m(3, 0) * m(1, 2), c19 = m(1, 0) * m(2, 2) - m(2, 0) * m(1, 2);
+  const double c20 = m(2, 0) * m(3, 1) - m(3, 0) * m(2, 1), c22 = m(1, 0) * m(3, 1) - m(3, 0) * m(1, 1), c23 = m(1, 0) * m(2, 1) - m(2, 0) * m(1, 1);
+  const double fac[6][4] = {{c00, c00, c02, c03}, {c04, c04, c06, c07}, {c08, c08, c10, c11},
+                            {c12, c12, c14, c15}, {c16, c16, c18, c19}, {c20, c20, c22, c23}};
+  double vec[4][4];   // Vec0..Vec3 = (m[1][r], m[0][r], m[0][r], m[0][r]) for r = 0..3
+  for (int r = 0; r < 4; ++r) { vec[r][0] = m(1, r); vec[r][1] = vec[r][2] = vec[r][3] = m(0, r); }
+  // Inv0 = V1 F0 - V2 F1 + V3 F2;  Inv1 = V0 F0 - V2 F3 + V3 F4;  Inv2 = V0 F1 - V1 F3 + V3 F5;  Inv3 = V0 F2 - V1 F4 + V2 F5
+  static const int terms[4][6] = {{1, 0, 2, 1, 3, 2}, {0, 0, 2, 3, 3, 4}, {0, 1, 1, 3, 3, 5}, {0, 2, 1, 4, 2, 5}};
+  double inv[16];
+  for (int c = 0; c < 4; ++c) {
+    const int* t = terms[c];
+    const double sign0 = (c & 1) ? -1.0 : 1.0;   // SignA = (+,-,+,-) for columns 0 and 2, SignB = (-,+,-,+) for 1 and 3
+    for (int k = 0; k < 4; ++k) {
+      const double v = (vec[t[0]][k] * fac[t[1]][k] - vec[t[2]][k] * fac[t[3]][k]) + vec[t[4]][k] * fac[t[5]][k];
+      inv[c * 4 + k] = v * ((k & 1) ? -sign0 : sign0);
+    }
+  }
+  const double d0 = m(0, 0) * inv[0], d1 = m(0, 1) * inv[4], d2 = m(0, 2) * inv[8], d3 = m(0, 3) * inv[12];
+  const double one_over_det = 1.0 / ((d0 + d1) + (d2 + d3));
+  for (int k = 0; k < 16; ++k) out[k] = inv[k] * one_over_det;
+}
+
+// InvVP = ModelMatrix * inverse(ProjectionMatrix * ModelViewMatrix): clip space -> world space, in double from the float
+// uniforms, rounded to float once per element
+static void voxel_view_matrix(const Params& P, float* inv_vp) {
+  double model[16], mv[16], proj[16], pmv[16], ipmv[16], r[16];
+  for (int k = 0; k < 16; ++k) { model[k] = P.model[k]; mv[k] = P.model_view[k]; proj[k] = P.proj[k]; }
+  mat4_mul(proj, mv, pmv);
+  mat4_inverse_glm(pmv, ipmv);
+  mat4_mul(model, ipmv, r);
+  for (int k = 0; k < 16; ++k) inv_vp[k] = (float)r[k];
+}
+
+int vct_render_voxels(vct_handle c, int level, uint8_t* host_rgba, uint32_t* host_voxel) {
+  NEED(c);
+  int rc = ensure_grid(c); if (rc) return rc;
+  if (level < 0 || level >= c->P.levels) return set_error(c, VCT_ERR_INVALID, "vct_render_voxels: level outside [0, levels)");
+  if (level > 0 && !c->grid[c->cur].mips_current)
+    return set_error(c, VCT_ERR_STATE, "vct_render_voxels: the mip levels are stale (call vct_build_mips after vct_upload_grid_level0)");
+  rc = ensure_frame(c); if (rc) return rc;
+  float inv_vp[16];
+  voxel_view_matrix(c->P, inv_vp);
+  const size_t n = (size_t)c->P.W * c->P.H;
+  uint32_t* d_voxel = nullptr;
+  if (host_voxel) VCT_CUDA(c, cudaMalloc(&d_voxel, n * 4));
+  rc = launch_voxel_view(c, level, inv_vp, d_voxel);
+  cudaError_t e = cudaSuccess;
+  if (!rc && host_rgba) e = cudaMemcpyAsync(host_rgba, c->d_frame, n * 4, cudaMemcpyDeviceToHost, c->stream);
+  if (!rc && host_voxel && e == cudaSuccess) e = cudaMemcpyAsync(host_voxel, d_voxel, n * 4, cudaMemcpyDeviceToHost, c->stream);
+  if (!rc && (host_rgba || host_voxel) && e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
+  if (d_voxel) { if (rc || e != cudaSuccess) cudaStreamSynchronize(c->stream); cudaFree(d_voxel); }
+  if (rc) return rc;
+  return check_cuda(c, e, "vct_render_voxels");
+}
+
 static int ensure_overlap(vct_context* c) {
   if (!c->stream2) {
     // higher priority than the main stream: cone_trace fills the machine with ~32 K small blocks, and the block
@@ -1199,6 +1271,14 @@ int vct_fragment_count(vct_handle c, uint64_t* n) {
 }
 int vct_debug_counter(vct_handle c, int which, uint64_t* n) {   /* 0 = work items of the last raster pass */
   NEED(c);
+  if (which == 1) {                                              /* texels the last voxel view visited */
+    unsigned long long parts[64 * 4];
+    int rc = read_counter(c, c->d_counters->view_steps, parts, sizeof(parts));
+    unsigned long long s = 0;
+    for (int k = 0; k < 64; ++k) s += parts[k * 4];
+    if (n) *n = s;
+    return rc;
+  }
   unsigned int v = 0;
   int rc = read_counter(c, which == 0 ? (const void*)&c->d_counters->n_items : (const void*)&c->d_counters->overflow, &v, 4);
   if (n) *n = v;

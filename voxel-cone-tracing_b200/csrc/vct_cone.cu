@@ -388,12 +388,6 @@ __device__ __forceinline__ void march_pixel(cudaTextureObject_t grid, const Para
   specular = make_float4(sr, sg, sb, socc);
 }
 
-__device__ __forceinline__ unsigned char to_unorm8(float x) {
-  x = fminf(fmaxf(x, 0.0f), 1.0f);
-  if (!(x == x)) x = 0.0f;
-  return (unsigned char)__float2int_rn(x * 255.0f);
-}
-
 // one warp = 8x4 pixels; block = 2 warps = 8x8 pixels (small blocks: the specular chain length varies a lot
 // between warps and a block holds its registers until its slowest warp is done)
 constexpr int BT = 64;

@@ -70,6 +70,9 @@ struct Counters {
   // executed textureLod calls of the last cone_trace: 64 partial counters, one 32-byte sector each (65 K warps adding
   // into ONE address serialise in a single L2 atomic unit); vct_cone_samples sums them
   unsigned long long cone_samples[64 * 4];
+  // texels visited by the last voxel view (vct_debug_counter 1), partial counters as above.  Appended last so that no
+  // field the other kernels address moves.
+  unsigned long long view_steps[64 * 4];
 };
 
 // Per-vertex transform cache written once per frame by vertex_pass -- the vertex-shader stage of the three
@@ -242,6 +245,7 @@ int launch_mip(vct_context* c);
 int launch_visibility(vct_context* c);
 int launch_cone(vct_context* c);
 int launch_reinject(vct_context* c);
+int launch_voxel_view(vct_context* c, int level, const float inv_vp[16], uint32_t* d_voxel);   // vct_view.cu
 int check_overflow(vct_context* c);
 int comm_barrier(vct_context* c, int channel, cudaStream_t stream);   // device-side cross-rank barrier, in stream order
 int comm_check(vct_context* c);                                        // barrier time-outs -> VCT_ERR_STATE
@@ -549,6 +553,13 @@ __device__ __forceinline__ float lod_from_derivs(float dudx, float dvdx, float d
   float rho2 = fmaxf(ax * ax + bx * bx, ay * ay + by * by);
   if (!(rho2 > 0.0f)) return 0.0f;
   return 0.5f * __log2f(rho2);
+}
+
+// float colour -> unorm8 (GL's conversion of a fragment output to an RGBA8 attachment)
+__device__ __forceinline__ unsigned char to_unorm8(float x) {
+  x = fminf(fmaxf(x, 0.0f), 1.0f);
+  if (!(x == x)) x = 0.0f;
+  return (unsigned char)__float2int_rn(x * 255.0f);
 }
 
 __device__ __forceinline__ float4 sample_material(cudaTextureObject_t t, float u, float v, float lod) {

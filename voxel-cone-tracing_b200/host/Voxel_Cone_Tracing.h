@@ -155,6 +155,12 @@ struct Voxel_Cone_Tracing {
     check(vct_render(device, host_rgba));      // model.Draw(VoxelConeTracingShader)
   }
 
+  // voxel view (no reference counterpart): mip `level` of the voxel pyramid drawn as cubes from the camera of Render()
+  void RenderVoxels(int level, uint8_t* host_rgba = nullptr) {
+    SetRenderUniforms();
+    check(vct_render_voxels(device, level, host_rgba, nullptr));
+  }
+
   // the uniform block of Render() (Voxel_Cone_Tracing.h:161-187), separated so that a sharded frame can set it too
   void SetRenderUniforms() {
     mat4 vMat = camera.GetViewMatrix();

@@ -3,7 +3,8 @@
 // Needs a CUDA device to run; compiling and linking it is part of build().
 //   facade_demo [dump_dir]   with a directory: also writes the flattened scene (verts.f32, idx.u32, trimat.u16), the
 //   uniforms of every frame (uniforms_<f>.f32: ModelView, Projection, DepthMVP, ProjX, ProjY, ProjZ, camera) and the
-//   frames (frame_<f>.rgba), so that a test can replay the same inputs through another binding and compare bytes.
+//   frames (frame_<f>.rgba) and voxel views of mip level 1 (voxels_<f>.rgba), so that a test can replay the same inputs
+//   through another binding and compare bytes.
 //   facade_demo <dump_dir> sharded [second_device]   also renders the views as sharded frames over two ranks.
 #include <cstdio>
 #include <cstdlib>
@@ -61,7 +62,7 @@ int main(int argc, char** argv) {
       dump(dir + "idx.u32", m.indices.data(), m.indices.size() * sizeof(unsigned));
       dump(dir + "trimat.u16", m.triangle_material.data(), m.triangle_material.size() * sizeof(uint16_t));
     }
-    std::vector<uint8_t> frame(256 * 256 * 4);
+    std::vector<uint8_t> frame(256 * 256 * 4), view(256 * 256 * 4);
     for (int f = 0; f < 3; ++f) {
       camera.Yaw = -90.0f + 2.0f * f;
       voxel_cone_tracing.Render(frame.data());
@@ -79,6 +80,8 @@ int main(int argc, char** argv) {
         u.push_back(camera.position.x); u.push_back(camera.position.y); u.push_back(camera.position.z);
         dump(dir + "uniforms_" + std::to_string(f) + ".f32", u.data(), u.size() * sizeof(float));
         dump(dir + "frame_" + std::to_string(f) + ".rgba", frame.data(), frame.size());
+        voxel_cone_tracing.RenderVoxels(1, view.data());
+        dump(dir + "voxels_" + std::to_string(f) + ".rgba", view.data(), view.size());
       }
     }
     // The same three views as ONE sharded frame stream over two ranks (two GPUs if the machine has them, else two

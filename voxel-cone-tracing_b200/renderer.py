@@ -151,6 +151,12 @@ class Voxel_Cone_Tracing:
         self._set_render_uniforms()
         self.ctx.render(out)
 
+    def RenderVoxels(self, level, out=None):
+        """Voxel view (no reference counterpart): mip `level` of the current pyramid drawn as cubes from the camera of
+        Render, into the frame buffer and, if given, `out`."""
+        self._set_render_uniforms()
+        self.ctx.render_voxels(level, out)
+
     def Frame(self, out=None):
         """DrawVoxelTexture + Render in one call (what 'full frames/s' times)."""
         self._set_render_uniforms()
