@@ -45,7 +45,8 @@ typedef enum vct_pass {
   VCT_PASS_EXCHANGE_PUSH = 10,  /* vct_voxelize_shared: multicast of the touched voxels (multimem.st / multimem.red) */
   VCT_PASS_EXCHANGE_MERGE = 11, /* vct_resolve_shared (inbox): the other ranks' records added to the accumulator     */
   VCT_PASS_VOXEL_VIEW = 12, /* vct_render_voxels (no reference counterpart)                          */
-  VCT_PASS_COUNT = 13
+  VCT_PASS_PROBES = 13,     /* vct_bake_probes (no reference counterpart)                            */
+  VCT_PASS_COUNT = 14
 } vct_pass;
 
 /* ---- lifetime.  Replaces Voxel_Cone_Tracing::Voxel_Cone_Tracing + init_voxel_cone_tracing resource
@@ -217,7 +218,8 @@ int vct_frame_buffer(vct_handle h, void** device_ptr, size_t* n_bytes);
 int vct_cone_samples(vct_handle h, uint64_t* n);       /* textureLod calls of the last vct_render */
 int vct_fragment_count(vct_handle h, uint64_t* n);     /* fragments of the last voxelisation */
 int vct_occupied_voxels(vct_handle h, uint64_t* n);
-/* diagnostics: 0 = tile work items of the last raster pass, 1 = texels the last voxel view visited (all pixels) */
+/* diagnostics: 0 = tile work items of the last raster pass, 1 = texels the last voxel view visited (all pixels),
+ * 2 = textureLod calls of the last vct_bake_probes (all probes and faces) */
 int vct_debug_counter(vct_handle h, int which, uint64_t* n);
 
 /* ---- cone queries: Voxel_Cone_Tracing(direction, tanHalfAngle) (VoxelConeTracing.fs:82-107) for arbitrary
@@ -226,6 +228,21 @@ int vct_debug_counter(vct_handle h, int which, uint64_t* n);
  * exercise the hardware-filtered tex3DLod path sample by sample. */
 int vct_trace_cones(vct_handle h, size_t n, const float* starts, const float* dirs, const float* tan_half,
                     float* out_rgb_occ, uint32_t* out_steps);
+
+/* Irradiance probes (no reference counterpart): the frame's diffuse term -- indirect light ind.rgb and occlusion,
+ * VoxelConeTracing.fs:196-201 -- at n points p (xyz n*3, world space as Position_world) for a surface facing each of
+ * +X, -X, +Y, -Y, +Z, -Z in that order.  Face f turns the current cone table (vct_set_cones) by a fixed orthonormal basis
+ * (T, B, N) with N the face's axis, starts at p + N * VoxelGridWorldSize / VoxelDimensions and marches every cone as
+ * vct_trace_cones does with DiffuseTanHalfAngle, weighted sum in cone order.  out[((p*6)+f)*4 + k] = (ind.r, ind.g,
+ * ind.b, 1 - ind.a); steps[p*6+f] (may be NULL) = textureLod calls of that face.  A probe with a non-finite coordinate
+ * gives NaN and 0 steps.  Camera, screen size and row-sharding uniforms have no effect.  With on_device != 0 all
+ * pointers are device pointers on the context's device and the call is asynchronous on the context's stream (no
+ * allocation, no synchronisation); otherwise they are host arrays and the call returns when they are filled.  Reads the
+ * current pyramid after the frames issued before it and keeps a later frame from overwriting it while it runs; the frame
+ * buffer and vct_cone_samples are untouched.  n = 0: no-op.  VCT_ERR_INVALID: NULL xyz or out with n > 0, n too large;
+ * VCT_ERR_STATE: mip levels stale (vct_upload_grid_level0 without vct_build_mips).  DESIGN.md section 3 "Irradiance
+ * probes". */
+int vct_bake_probes(vct_handle h, size_t n, const float* xyz, float* out, uint32_t* steps, int on_device);
 
 /* SampleVoxels(World_Position, lod) (VoxelConeTracing.fs:59-66) for n points: pos n*3, lod n, out n*4 */
 int vct_sample_voxels(vct_handle h, size_t n, const float* world_pos, const float* lod, float* out_rgba);

@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(HERE, "lib", "libvct_b200.so")
 
 PASSES = {"depth": 0, "vox_clear": 1, "vox_cover": 2, "vox_shade": 3, "resolve": 4, "mip": 5,
           "visibility": 6, "cone": 7, "frame": 8, "reinject": 9, "exchange_push": 10, "exchange_merge": 11,
-          "voxel_view": 12}
+          "voxel_view": 12, "probes": 13}
 
 # every symbol include/vct_c_api.h declares (tests check the library exports all of them)
 SYMBOLS = [
@@ -24,7 +24,7 @@ SYMBOLS = [
     "vct_voxelize_shared", "vct_resolve_shared", "vct_frame_shared_begin", "vct_exchange_stream", "vct_frame_shared_end", "vct_readback_depth", "vct_readback_counts",
     "vct_readback_sums", "vct_readback_grid", "vct_upload_grid_level0", "vct_build_mips", "vct_readback_visibility",
     "vct_readback_frame", "vct_frame_buffer", "vct_cone_samples", "vct_fragment_count", "vct_occupied_voxels", "vct_debug_counter",
-    "vct_trace_cones", "vct_sample_voxels", "vct_set_stream", "vct_use_own_stream", "vct_sync", "vct_pass_time_us", "vct_kernel_launches", "vct_bench_tex3d",
+    "vct_trace_cones", "vct_bake_probes", "vct_sample_voxels", "vct_set_stream", "vct_use_own_stream", "vct_sync", "vct_pass_time_us", "vct_kernel_launches", "vct_bench_tex3d",
     "vct_bench_tex3d_format", "vct_bench_atomics", "vct_pass_timeline",
     "vct_comm_init", "vct_comm_destroy", "vct_comm_info", "vct_comm_barrier", "vct_frame_sharded", "vct_frame_sharded_wait",
     "vct_comm_frame_buffer", "vct_create_multi", "vct_comm_init_multi", "vct_frame_sharded_multi",
@@ -74,7 +74,7 @@ def load_library(path=None):
         "vct_readback_visibility": [vp, vp], "vct_readback_frame": [vp, vp],
         "vct_frame_buffer": [vp, C.POINTER(vp), C.POINTER(sz)], "vct_cone_samples": [vp, C.POINTER(C.c_uint64)],
         "vct_fragment_count": [vp, C.POINTER(C.c_uint64)], "vct_occupied_voxels": [vp, C.POINTER(C.c_uint64)], "vct_debug_counter": [vp, i, C.POINTER(C.c_uint64)],
-        "vct_trace_cones": [vp, sz, vp, vp, vp, vp, vp], "vct_sample_voxels": [vp, sz, vp, vp, vp], "vct_set_stream": [vp, vp], "vct_use_own_stream": [vp], "vct_sync": [vp], "vct_pass_time_us": [vp, i, C.POINTER(f)],
+        "vct_trace_cones": [vp, sz, vp, vp, vp, vp, vp], "vct_bake_probes": [vp, sz, vp, vp, vp, i], "vct_sample_voxels": [vp, sz, vp, vp, vp], "vct_set_stream": [vp, vp], "vct_use_own_stream": [vp], "vct_sync": [vp], "vct_pass_time_us": [vp, i, C.POINTER(f)],
         "vct_kernel_launches": [vp, C.POINTER(C.c_uint64)],
         "vct_bench_tex3d": [vp, i, C.c_uint64, i, f, i, C.POINTER(f)],
         "vct_bench_tex3d_format": [vp, i, i, C.c_uint64, i, f, i, C.POINTER(f)],
@@ -384,6 +384,28 @@ class Context:
         out = np.empty((s.shape[0], 4), dtype=np.float32)
         steps = np.empty(s.shape[0], dtype=np.uint32)
         self._ck(self.L.vct_trace_cones(self.h, s.shape[0], _ptr(s), _ptr(d), _ptr(t), _ptr(out), _ptr(steps)))
+        return out, steps
+
+    def bake_probes(self, xyz=None, out=None, steps=None, n=None, device_xyz=None, device_out=None, device_steps=None):
+        """Irradiance probes: indirect light and occlusion at each point for a surface facing +X, -X, +Y, -Y, +Z, -Z.
+
+        Host form: `xyz` (n, 3) float32; returns `out` (n, 6, 4) float32 = (r, g, b, occlusion) per face and `steps`
+        (n, 6) uint32 textureLod calls per face (both allocated unless given).  Device form: `n` probes at the device
+        pointers `device_xyz` (n*3 float32), `device_out` (n*24 float32) and optionally `device_steps` (n*6 uint32), e.g.
+        torch CUDA tensors' data_ptr(); asynchronous on the context's stream, returns None."""
+        if device_xyz is not None or device_out is not None:
+            ptr = lambda p: None if p is None else C.c_void_p(int(p))
+            self._ck(self.L.vct_bake_probes(self.h, int(n), ptr(device_xyz), ptr(device_out), ptr(device_steps), 1))
+            return None
+        x = np.ascontiguousarray(xyz, dtype=np.float32).reshape(-1, 3)
+        k = x.shape[0]
+        if out is None:
+            out = np.empty((k, 6, 4), dtype=np.float32)
+        if steps is None:
+            steps = np.empty((k, 6), dtype=np.uint32)
+        assert out.dtype == np.float32 and out.flags.c_contiguous and out.size == k * 24
+        assert steps.dtype == np.uint32 and steps.flags.c_contiguous and steps.size == k * 6
+        self._ck(self.L.vct_bake_probes(self.h, k, _ptr(x), _ptr(out), _ptr(steps), 0))
         return out, steps
 
     # ---- execution control

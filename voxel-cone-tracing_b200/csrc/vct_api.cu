@@ -513,6 +513,7 @@ int vct_destroy(vct_handle c) {
   cudaFree(c->mask_prev[0]); cudaFree(c->mask_prev[1]); cudaFree(c->d_push_list); cudaFree(c->d_push_count);
   cudaFree(c->d_voxrec); cudaFree(c->d_depth); cudaFree(c->d_frags); cudaFree(c->d_items); cudaFree(c->d_counters);
   cudaFree(c->d_vis2[0]); cudaFree(c->d_vis2[1]); cudaFree(c->d_frame);
+  cudaFree(c->d_probe_buf);
   for (int k = 0; k < 2; ++k) if (c->slot_read_done[k]) cudaEventDestroy(c->slot_read_done[k]);
   if (c->stream_vox) { cudaStreamDestroy(c->stream_vox); cudaEventDestroy(c->ev_vox_done); cudaEventDestroy(c->ev_vtx_done); }
   for (int k = 0; k < 3; ++k) { cudaFree(c->d_frame2[k]); if (c->ev_rendered[k]) cudaEventDestroy(c->ev_rendered[k]); if (c->ev_copied[k]) cudaEventDestroy(c->ev_copied[k]); }
@@ -1271,9 +1272,9 @@ int vct_fragment_count(vct_handle c, uint64_t* n) {
 }
 int vct_debug_counter(vct_handle c, int which, uint64_t* n) {   /* 0 = work items of the last raster pass */
   NEED(c);
-  if (which == 1) {                                              /* texels the last voxel view visited */
+  if (which == 1 || which == 2) {       /* texels the last voxel view visited, textureLod calls of the last probe bake */
     unsigned long long parts[64 * 4];
-    int rc = read_counter(c, c->d_counters->view_steps, parts, sizeof(parts));
+    int rc = read_counter(c, which == 1 ? c->d_counters->view_steps : c->d_counters->probe_steps, parts, sizeof(parts));
     unsigned long long s = 0;
     for (int k = 0; k < 64; ++k) s += parts[k * 4];
     if (n) *n = s;
@@ -1298,6 +1299,38 @@ int vct_trace_cones(vct_handle c, size_t n, const float* starts, const float* di
   NEED(c);
   if (n && (!starts || !dirs || !tans || !out)) return set_error(c, VCT_ERR_INVALID, "vct_trace_cones: null argument");
   return trace_cones(c, n, starts, dirs, tans, out, steps);
+}
+
+int vct_bake_probes(vct_handle c, size_t n, const float* xyz, float* out, uint32_t* steps, int on_device) {
+  NEED(c);
+  if (!n) return VCT_OK;
+  if (!xyz || !out) return set_error(c, VCT_ERR_INVALID, "vct_bake_probes: null argument");
+  if (n > SIZE_MAX / 256) return set_error(c, VCT_ERR_INVALID, "vct_bake_probes: n too large");
+  int rc = ensure_grid(c); if (rc) return rc;
+  if (!c->grid[c->cur].mips_current)   // every cone reads every level
+    return set_error(c, VCT_ERR_STATE, "vct_bake_probes: the mip levels are stale (call vct_build_mips after vct_upload_grid_level0)");
+  if (on_device) return launch_probes(c, n, xyz, out, steps);
+  // host arrays: staged through one device buffer kept on the context (the previous host-form bake has completed)
+  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  const size_t b_xyz = n * 12, b_out = n * 96, b_steps = steps ? n * 24 : 0;
+  const size_t need = up(b_xyz) + up(b_out) + b_steps;
+  if (c->probe_buf_bytes < need) {
+    cudaFree(c->d_probe_buf);
+    c->d_probe_buf = nullptr; c->probe_buf_bytes = 0;
+    VCT_CUDA(c, cudaMalloc(&c->d_probe_buf, need));
+    c->probe_buf_bytes = need;
+  }
+  float* d_xyz = (float*)c->d_probe_buf;
+  float* d_out = (float*)(c->d_probe_buf + up(b_xyz));
+  uint32_t* d_steps = steps ? (uint32_t*)(c->d_probe_buf + up(b_xyz) + up(b_out)) : nullptr;
+  VCT_CUDA(c, cudaMemcpyAsync(d_xyz, xyz, b_xyz, cudaMemcpyHostToDevice, c->stream));
+  rc = launch_probes(c, n, d_xyz, d_out, d_steps);
+  cudaError_t e = cudaSuccess;
+  if (!rc) e = cudaMemcpyAsync(out, d_out, b_out, cudaMemcpyDeviceToHost, c->stream);
+  if (!rc && steps && e == cudaSuccess) e = cudaMemcpyAsync(steps, d_steps, b_steps, cudaMemcpyDeviceToHost, c->stream);
+  cudaError_t es = cudaStreamSynchronize(c->stream);   // the staging buffer is free again when this returns
+  if (rc) return rc;
+  return check_cuda(c, e != cudaSuccess ? e : es, "vct_bake_probes");
 }
 
 // ---- execution control

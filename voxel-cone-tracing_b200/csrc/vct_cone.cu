@@ -673,6 +673,73 @@ int trace_cones(vct_context* c, size_t n, const float* starts, const float* dirs
   return check_cuda(c, e, "vct_trace_cones");
 }
 
+// Irradiance probes (vct_bake_probes, no reference counterpart): the frame's diffuse term (VoxelConeTracing.fs:92,
+// :196-201) at caller-supplied points, for a surface facing each of +X, -X, +Y, -Y, +Z, -Z (DESIGN.md section 3
+// "Irradiance probes").  One thread per (probe, face); blockIdx.y is the face, so the block's rotated cone directions
+// are computed once into shared memory, and consecutive threads take consecutive probes.  Every cone is cone_march, as
+// in trace_cones_kernel: a probe equals the float32 composition of vct_trace_cones bit for bit.
+constexpr int PROBE_BT = 128;
+struct ProbeBasis { float tbn[6][9]; };   // per face: T, B, N
+
+__global__ void __launch_bounds__(PROBE_BT) bake_probes_kernel(Params P, ProbeBasis basis, cudaTextureObject_t grid,
+                                                               size_t n, const float* __restrict__ xyz,
+                                                               float* __restrict__ out, uint32_t* __restrict__ steps,
+                                                               Counters* __restrict__ ctr) {
+  __shared__ float s_dir[VCT_MAX_CONES * 3];
+  const int face = blockIdx.y;
+  const float* tbn = basis.tbn[face];
+  const int nc = min(P.n_cones, VCT_MAX_CONES);
+  if ((int)threadIdx.x < nc) {
+    // d.x T + d.y B + d.z N: one non-zero term per component (a signed permutation of d), so the sum is exact
+    const float* d = &P.cone_dir[threadIdx.x * 3];
+    const V3 dir = vnormalize(v3((d[0] * tbn[0] + d[1] * tbn[3]) + d[2] * tbn[6], (d[0] * tbn[1] + d[1] * tbn[4]) + d[2] * tbn[7],
+                                 (d[0] * tbn[2] + d[1] * tbn[5]) + d[2] * tbn[8]));
+    s_dir[threadIdx.x * 3] = dir.x; s_dir[threadIdx.x * 3 + 1] = dir.y; s_dir[threadIdx.x * 3 + 2] = dir.z;
+  }
+  __syncthreads();
+  const size_t p = (size_t)blockIdx.x * PROBE_BT + threadIdx.x;
+  unsigned cnt = 0;
+  if (p < n) {
+    const float x = xyz[3 * p], y = xyz[3 * p + 1], z = xyz[3 * p + 2];
+    float4 r = make_float4(NAN, NAN, NAN, NAN);
+    if (isfinite(x) && isfinite(y) && isfinite(z)) {
+      const ConeConsts kc = cone_consts(P);
+      const V3 start = vadd(v3(x, y, z), vscale(v3(tbn[6], tbn[7], tbn[8]), kc.vws));   // :92
+      float ir = 0.0f, ig = 0.0f, ib = 0.0f, ia = 0.0f;
+#pragma unroll 1
+      for (int c = 0; c < nc; ++c) {
+        const float4 s = cone_march(grid, P, kc, start, v3(s_dir[c * 3], s_dir[c * 3 + 1], s_dir[c * 3 + 2]), P.diffuse_tan, cnt);
+        const float w = P.cone_w[c];
+        ir = ir + w * s.x; ig = ig + w * s.y; ib = ib + w * s.z; ia = ia + w * s.w;
+      }
+      r = make_float4(ir, ig, ib, 1.0f - ia);                                              // ind.rgb, occlusion (:201)
+    }
+    float* o = out + (p * 6 + face) * 4;
+    o[0] = r.x; o[1] = r.y; o[2] = r.z; o[3] = r.w;
+    if (steps) steps[p * 6 + face] = cnt;
+  }
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, d);
+  if ((threadIdx.x & 31) == 0 && cnt)
+    atomicAdd(&ctr->probe_steps[((blockIdx.x + blockIdx.y * 7u) & 63u) * 4], (unsigned long long)cnt);
+}
+
+int launch_probes(vct_context* c, size_t n, const float* xyz, float* out, uint32_t* steps) {
+  // DESIGN.md section 3: each row right-handed and orthonormal, faces +X, -X, +Y, -Y, +Z, -Z
+  static const ProbeBasis basis = {{{0, 0, -1, 0, 1, 0, 1, 0, 0}, {0, 0, 1, 0, 1, 0, -1, 0, 0},
+                                    {1, 0, 0, 0, 0, -1, 0, 1, 0}, {1, 0, 0, 0, 0, 1, 0, -1, 0},
+                                    {1, 0, 0, 0, 1, 0, 0, 0, 1}, {-1, 0, 0, 0, 1, 0, 0, 0, -1}}};
+  const size_t blocks = (n + PROBE_BT - 1) / PROBE_BT;
+  if (blocks > 0x7fffffffu) return set_error(c, VCT_ERR_INVALID, "vct_bake_probes: too many probes for one launch");
+  PassTimer timer(c, VCT_PASS_PROBES);
+  VCT_CUDA(c, cudaMemsetAsync(c->d_counters->probe_steps, 0, sizeof(c->d_counters->probe_steps), c->stream));
+  bake_probes_kernel<<<dim3((unsigned)blocks, 6), PROBE_BT, 0, c->stream>>>(c->P, basis, c->grid[c->cur].tex, n, xyz, out,
+                                                                             steps, c->d_counters);
+  c->launches += 1;
+  mark_slot_read(c);
+  return check_cuda(c, cudaGetLastError(), "bake_probes");
+}
+
 __global__ void sample_voxels_kernel(Params P, cudaTextureObject_t grid, size_t n, const float* __restrict__ pos,
                                      const float* __restrict__ lod, float4* __restrict__ out) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;

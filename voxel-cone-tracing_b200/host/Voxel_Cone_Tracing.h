@@ -161,6 +161,12 @@ struct Voxel_Cone_Tracing {
     check(vct_render_voxels(device, level, host_rgba, nullptr));
   }
 
+  // irradiance probes (no reference counterpart): indirect light and occlusion of the current pyramid at n world points
+  // (xyz: n*3) for a surface facing +X, -X, +Y, -Y, +Z, -Z; out: n*6*4 (r, g, b, occlusion), steps: n*6 or NULL
+  void BakeProbes(const float* xyz, size_t n, float* out, uint32_t* steps = nullptr) {
+    check(vct_bake_probes(device, n, xyz, out, steps, 0));
+  }
+
   // the uniform block of Render() (Voxel_Cone_Tracing.h:161-187), separated so that a sharded frame can set it too
   void SetRenderUniforms() {
     mat4 vMat = camera.GetViewMatrix();

@@ -3,8 +3,9 @@
 // Needs a CUDA device to run; compiling and linking it is part of build().
 //   facade_demo [dump_dir]   with a directory: also writes the flattened scene (verts.f32, idx.u32, trimat.u16), the
 //   uniforms of every frame (uniforms_<f>.f32: ModelView, Projection, DepthMVP, ProjX, ProjY, ProjZ, camera) and the
-//   frames (frame_<f>.rgba) and voxel views of mip level 1 (voxels_<f>.rgba), so that a test can replay the same inputs
-//   through another binding and compare bytes.
+//   frames (frame_<f>.rgba), voxel views of mip level 1 (voxels_<f>.rgba) and, after the frames, the irradiance probes
+//   of the cell centres of an 8x8x8 lattice over the grid (probe_xyz.f32, probes.f32), so that a test can replay the
+//   same inputs through another binding and compare bytes.
 //   facade_demo <dump_dir> sharded [second_device]   also renders the views as sharded frames over two ranks.
 #include <cstdio>
 #include <cstdlib>
@@ -83,6 +84,21 @@ int main(int argc, char** argv) {
         voxel_cone_tracing.RenderVoxels(1, view.data());
         dump(dir + "voxels_" + std::to_string(f) + ".rgba", view.data(), view.size());
       }
+    }
+    if (!dir.empty()) {
+      const int k = 8;
+      const float G = voxel_cone_tracing.VoxelGridWorldSize, cell = G / (float)k;
+      std::vector<float> xyz, probes((size_t)k * k * k * 6 * 4);
+      for (int z = 0; z < k; ++z)
+        for (int y = 0; y < k; ++y)
+          for (int x = 0; x < k; ++x) {
+            xyz.push_back(((float)x + 0.5f) * cell - 0.5f * G);
+            xyz.push_back(((float)y + 0.5f) * cell - 0.5f * G);
+            xyz.push_back(((float)z + 0.5f) * cell - 0.5f * G);
+          }
+      voxel_cone_tracing.BakeProbes(xyz.data(), (size_t)k * k * k, probes.data());
+      dump(dir + "probe_xyz.f32", xyz.data(), xyz.size() * sizeof(float));
+      dump(dir + "probes.f32", probes.data(), probes.size() * sizeof(float));
     }
     // The same three views as ONE sharded frame stream over two ranks (two GPUs if the machine has them, else two
     // handles on GPU 0): the frames must equal the single-GPU ones byte for byte.

@@ -157,6 +157,13 @@ class Voxel_Cone_Tracing:
         self._set_render_uniforms()
         self.ctx.render_voxels(level, out)
 
+    def BakeProbes(self, xyz):
+        """Irradiance probes (no reference counterpart): indirect light and occlusion of the current pyramid at the
+        (n, 3) world points `xyz` for a surface facing +X, -X, +Y, -Y, +Z, -Z, with the cone table of Render.  Returns
+        (n, 6, 4) float32 (r, g, b, occlusion) and (n, 6) uint32 textureLod calls."""
+        self._set_render_uniforms()
+        return self.ctx.bake_probes(xyz)
+
     def Frame(self, out=None):
         """DrawVoxelTexture + Render in one call (what 'full frames/s' times)."""
         self._set_render_uniforms()
