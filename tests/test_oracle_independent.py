@@ -55,8 +55,9 @@ def sample_voxels(levels, pos, lod):
     return a
 
 
-def cone(levels, V, start, direction, tan_half, max_dist=75.0, max_alpha=0.95):
-    """VoxelConeTracing.fs:82-107 in float64; also returns how close alpha came to the exit threshold."""
+def cone(levels, V, start, direction, tan_half, max_dist=75.0, max_alpha=0.95, step_mult=1.0):
+    """VoxelConeTracing.fs:82-107 in float64 (the step is diameter * StepMultiplier, 1 in the reference); also returns
+    how close alpha and distance came to their exit thresholds."""
     vws = G / V
     dist, alpha, occ, color, n, margin = vws, 0.0, 0.0, np.zeros(3), 0, 1.0
     start, direction = np.asarray(start, dtype=np.float64), np.asarray(direction, dtype=np.float64)
@@ -66,7 +67,7 @@ def cone(levels, V, start, direction, tan_half, max_dist=75.0, max_alpha=0.95):
         color += (1 - alpha) * s[:3]
         occ += (1 - alpha) * s[3] / (1 + 0.03 * diameter)
         alpha += (1 - alpha) * s[3]
-        dist += diameter
+        dist += diameter * step_mult
         n += 1
         margin = min(margin, abs(alpha - max_alpha), abs(dist - max_dist) / max_dist)
     return np.append(color, occ), n, margin
@@ -344,9 +345,9 @@ def test_visibility_against_float64_ray_casting(oracle):
 
 
 # ------------------------------------------------------------------------------------- whole fragment shader
-def pcf_lit_taps(tex, S, dc, bias=0.002):
-    """Voxelization.fs:18-52 / VoxelConeTracing.fs:132-163 without the final normalisation; also says whether any tap
-    sits on the compare threshold."""
+def pcf_lit_taps(tex, S, dc, bias=0.002, r=2):
+    """Voxelization.fs:18-52 / VoxelConeTracing.fs:132-163 without the final normalisation, for a (2r+1)^2 tap kernel
+    (r = 2 in the reference); also says whether any tap sits on the compare threshold."""
     def bilinear(s, t):
         x, y = s * S - 0.5, t * S - 0.5
         i, j = int(np.floor(x)), int(np.floor(y))
@@ -356,8 +357,8 @@ def pcf_lit_taps(tex, S, dc, bias=0.002):
         return (1 - b) * ((1 - a) * at(i, j) + a * at(i + 1, j)) + b * ((1 - a) * at(i, j + 1) + a * at(i + 1, j + 1))
     cur = dc[2] / dc[3]
     lit, safe = 0, True
-    for x in range(-2, 3):
-        for y in range(-2, 3):
+    for x in range(-r, r + 1):
+        for y in range(-r, r + 1):
             closest = bilinear(dc[0] + x / S, dc[1] + y / S)
             safe &= abs((cur - bias) - closest) > 2e-6
             lit += (cur - bias) <= closest

@@ -25,15 +25,18 @@ REFERENCE_CONE_WEIGHTS = np.array([0.25, 0.15, 0.15, 0.15, 0.15, 0.15], dtype=np
 
 def cone_set(kind="6+1"):
     """'6+1' = the reference's table; '5+1' = BASELINE config 2 wording (the five 60-degree cones,
-    weights renormalised to 1); '9+1' = config 3 extension (normal + 8 at 60 degrees)."""
+    weights renormalised to 1); '9+1' = config 3 extension (normal + 8 at 60 degrees); '16+1' = the largest
+    table the library takes (normal at 0.1 + 15 at 60 degrees at 0.06 each)."""
     if kind == "6+1":
         return REFERENCE_CONE_DIRECTIONS.copy(), REFERENCE_CONE_WEIGHTS.copy()
     if kind == "5+1":
         return REFERENCE_CONE_DIRECTIONS[1:].copy(), np.full(5, 0.2, dtype=np.float32)
-    if kind == "9+1":
-        a = np.arange(8) * (2 * np.pi / 8)
-        d = np.concatenate([[[0, 0, 1]], np.stack([0.866025 * np.cos(a), 0.866025 * np.sin(a), np.full(8, 0.5)], 1)])
-        w = np.concatenate([[0.2], np.full(8, 0.1)])
+    ring = {"9+1": (8, 0.2, 0.1), "16+1": (15, 0.1, 0.06)}
+    if kind in ring:
+        n, w0, w1 = ring[kind]
+        a = np.arange(n) * (2 * np.pi / n)
+        d = np.concatenate([[[0, 0, 1]], np.stack([0.866025 * np.cos(a), 0.866025 * np.sin(a), np.full(n, 0.5)], 1)])
+        w = np.concatenate([[w0], np.full(n, w1)])
         return d.astype(np.float32), w.astype(np.float32)
     raise ValueError(kind)
 
