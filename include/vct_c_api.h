@@ -46,7 +46,8 @@ typedef enum vct_pass {
   VCT_PASS_EXCHANGE_MERGE = 11, /* vct_resolve_shared (inbox): the other ranks' records added to the accumulator     */
   VCT_PASS_VOXEL_VIEW = 12, /* vct_render_voxels (no reference counterpart)                          */
   VCT_PASS_PROBES = 13,     /* vct_bake_probes (no reference counterpart)                            */
-  VCT_PASS_COUNT = 14
+  VCT_PASS_RAYS = 14,       /* vct_cast_rays (no reference counterpart)                              */
+  VCT_PASS_COUNT = 15
 } vct_pass;
 
 /* ---- lifetime.  Replaces Voxel_Cone_Tracing::Voxel_Cone_Tracing + init_voxel_cone_tracing resource
@@ -219,7 +220,8 @@ int vct_cone_samples(vct_handle h, uint64_t* n);       /* textureLod calls of th
 int vct_fragment_count(vct_handle h, uint64_t* n);     /* fragments of the last voxelisation */
 int vct_occupied_voxels(vct_handle h, uint64_t* n);
 /* diagnostics: 0 = tile work items of the last raster pass, 1 = texels the last voxel view visited (all pixels),
- * 2 = textureLod calls of the last vct_bake_probes (all probes and faces) */
+ * 2 = textureLod calls of the last vct_bake_probes (all probes and faces), 3 = texels the last vct_cast_rays visited
+ * (all segments) */
 int vct_debug_counter(vct_handle h, int which, uint64_t* n);
 
 /* ---- cone queries: Voxel_Cone_Tracing(direction, tanHalfAngle) (VoxelConeTracing.fs:82-107) for arbitrary
@@ -243,6 +245,25 @@ int vct_trace_cones(vct_handle h, size_t n, const float* starts, const float* di
  * VCT_ERR_STATE: mip levels stale (vct_upload_grid_level0 without vct_build_mips).  DESIGN.md section 3 "Irradiance
  * probes". */
 int vct_bake_probes(vct_handle h, size_t n, const float* xyz, float* out, uint32_t* steps, int on_device);
+
+/* Ray casts (no reference counterpart): for each of n world-space segments a -> b (segments: n*6 floats a.xyz, b.xyz, in
+ * the space of Position_world / vct_bake_probes), the first occupied texel of mip `level` of the current pyramid.  The
+ * walk is the voxel view's (DESIGN.md section 3 "Voxel view" steps 3-5, "Ray casts") from o = (a/G + 0.5)*N to
+ * e = (b/G + 0.5)*N in texel space, N = VoxelDimensions >> level, G = VoxelGridWorldSize; the segment is t in [0, 1], the
+ * grid does not repeat.  Per segment on a hit: voxel = (z*N + y)*N + x; t = the segment parameter at which the walk
+ * entered that texel; face = the outward normal of the face it entered through, 1..6 = +X, -X, +Y, -Y, +Z, -Z, 0 when
+ * the segment starts inside it; rgba = its colour un-premultiplied as the view shows it before face shading, alpha = its
+ * alpha as unorm8; steps = texels visited.  On a miss: voxel 0xFFFFFFFF, t +inf, face 0, rgba 0.  a == b is a point
+ * query; a non-finite coordinate is a miss with 0 steps.  t, face, rgba (4 bytes per segment) and steps may be NULL.
+ * With on_device != 0 all pointers are device pointers on the context's device (rgba 4-byte aligned) and the call is
+ * asynchronous on the context's stream (no allocation, no synchronisation); otherwise they are host arrays and the call
+ * returns when they are filled.  Reads the current pyramid after the frames issued before it and keeps a later frame
+ * from overwriting it while it runs; the frame buffer and vct_cone_samples are untouched; the camera, screen size and
+ * row-sharding uniforms have no effect.  n = 0: no-op.  VCT_ERR_INVALID: level outside [0, levels), NULL segments or
+ * voxel with n > 0, n too large, a misaligned device rgba; VCT_ERR_STATE: level > 0 with the mip levels stale
+ * (vct_upload_grid_level0 without vct_build_mips). */
+int vct_cast_rays(vct_handle h, int level, size_t n, const float* segments, uint32_t* voxel, float* t, uint8_t* face,
+                  uint8_t* rgba, uint32_t* steps, int on_device);
 
 /* SampleVoxels(World_Position, lod) (VoxelConeTracing.fs:59-66) for n points: pos n*3, lod n, out n*4 */
 int vct_sample_voxels(vct_handle h, size_t n, const float* world_pos, const float* lod, float* out_rgba);

@@ -12,7 +12,7 @@ LIB_PATH = os.path.join(HERE, "lib", "libvct_b200.so")
 
 PASSES = {"depth": 0, "vox_clear": 1, "vox_cover": 2, "vox_shade": 3, "resolve": 4, "mip": 5,
           "visibility": 6, "cone": 7, "frame": 8, "reinject": 9, "exchange_push": 10, "exchange_merge": 11,
-          "voxel_view": 12, "probes": 13}
+          "voxel_view": 12, "probes": 13, "rays": 14}
 
 # every symbol include/vct_c_api.h declares (tests check the library exports all of them)
 SYMBOLS = [
@@ -24,7 +24,7 @@ SYMBOLS = [
     "vct_voxelize_shared", "vct_resolve_shared", "vct_frame_shared_begin", "vct_exchange_stream", "vct_frame_shared_end", "vct_readback_depth", "vct_readback_counts",
     "vct_readback_sums", "vct_readback_grid", "vct_upload_grid_level0", "vct_build_mips", "vct_readback_visibility",
     "vct_readback_frame", "vct_frame_buffer", "vct_cone_samples", "vct_fragment_count", "vct_occupied_voxels", "vct_debug_counter",
-    "vct_trace_cones", "vct_bake_probes", "vct_sample_voxels", "vct_set_stream", "vct_use_own_stream", "vct_sync", "vct_pass_time_us", "vct_kernel_launches", "vct_bench_tex3d",
+    "vct_trace_cones", "vct_bake_probes", "vct_cast_rays", "vct_sample_voxels", "vct_set_stream", "vct_use_own_stream", "vct_sync", "vct_pass_time_us", "vct_kernel_launches", "vct_bench_tex3d",
     "vct_bench_tex3d_format", "vct_bench_atomics", "vct_pass_timeline",
     "vct_comm_init", "vct_comm_destroy", "vct_comm_info", "vct_comm_barrier", "vct_frame_sharded", "vct_frame_sharded_wait",
     "vct_comm_frame_buffer", "vct_create_multi", "vct_comm_init_multi", "vct_frame_sharded_multi",
@@ -74,7 +74,7 @@ def load_library(path=None):
         "vct_readback_visibility": [vp, vp], "vct_readback_frame": [vp, vp],
         "vct_frame_buffer": [vp, C.POINTER(vp), C.POINTER(sz)], "vct_cone_samples": [vp, C.POINTER(C.c_uint64)],
         "vct_fragment_count": [vp, C.POINTER(C.c_uint64)], "vct_occupied_voxels": [vp, C.POINTER(C.c_uint64)], "vct_debug_counter": [vp, i, C.POINTER(C.c_uint64)],
-        "vct_trace_cones": [vp, sz, vp, vp, vp, vp, vp], "vct_bake_probes": [vp, sz, vp, vp, vp, i], "vct_sample_voxels": [vp, sz, vp, vp, vp], "vct_set_stream": [vp, vp], "vct_use_own_stream": [vp], "vct_sync": [vp], "vct_pass_time_us": [vp, i, C.POINTER(f)],
+        "vct_trace_cones": [vp, sz, vp, vp, vp, vp, vp], "vct_bake_probes": [vp, sz, vp, vp, vp, i], "vct_cast_rays": [vp, i, sz, vp, vp, vp, vp, vp, vp, i], "vct_sample_voxels": [vp, sz, vp, vp, vp], "vct_set_stream": [vp, vp], "vct_use_own_stream": [vp], "vct_sync": [vp], "vct_pass_time_us": [vp, i, C.POINTER(f)],
         "vct_kernel_launches": [vp, C.POINTER(C.c_uint64)],
         "vct_bench_tex3d": [vp, i, C.c_uint64, i, f, i, C.POINTER(f)],
         "vct_bench_tex3d_format": [vp, i, i, C.c_uint64, i, f, i, C.POINTER(f)],
@@ -407,6 +407,30 @@ class Context:
         assert steps.dtype == np.uint32 and steps.flags.c_contiguous and steps.size == k * 6
         self._ck(self.L.vct_bake_probes(self.h, k, _ptr(x), _ptr(out), _ptr(steps), 0))
         return out, steps
+
+    def cast_rays(self, level, segments=None, n=None, device_segments=None, device_voxel=None, device_t=None,
+                  device_face=None, device_rgba=None, device_steps=None):
+        """Ray casts: the first occupied texel of mip `level` along each world-space segment a -> b.
+
+        Host form: `segments` (n, 6) float32 (a.xyz, b.xyz); returns (voxel, t, face, rgba, steps): (n,) uint32 texel
+        indices (z*N + y)*N + x (0xFFFFFFFF = miss), (n,) float32 segment parameter where the walk entered the texel
+        (+inf = miss), (n,) uint8 entry-face normal 1..6 = +X, -X, +Y, -Y, +Z, -Z (0 = started inside it or missed),
+        (n, 4) uint8 un-premultiplied colour and alpha (0 = miss), (n,) uint32 texels visited.  Device form: `n`
+        segments at the device pointers `device_segments` (n*6 float32) and `device_voxel` (n uint32), optionally
+        `device_t`, `device_face`, `device_rgba` (n*4 bytes, 4-byte aligned) and `device_steps`, e.g. torch CUDA
+        tensors' data_ptr(); asynchronous on the context's stream, returns None."""
+        if device_segments is not None or device_voxel is not None:
+            ptr = lambda p: None if p is None else C.c_void_p(int(p))
+            self._ck(self.L.vct_cast_rays(self.h, int(level), int(n), ptr(device_segments), ptr(device_voxel), ptr(device_t),
+                                          ptr(device_face), ptr(device_rgba), ptr(device_steps), 1))
+            return None
+        s = np.ascontiguousarray(segments, dtype=np.float32).reshape(-1, 6)
+        k = s.shape[0]
+        voxel, t, face = np.empty(k, np.uint32), np.empty(k, np.float32), np.empty(k, np.uint8)
+        rgba, steps = np.empty((k, 4), np.uint8), np.empty(k, np.uint32)
+        self._ck(self.L.vct_cast_rays(self.h, int(level), k, _ptr(s), _ptr(voxel), _ptr(t), _ptr(face), _ptr(rgba),
+                                      _ptr(steps), 0))
+        return voxel, t, face, rgba, steps
 
     # ---- execution control
     def set_stream(self, cuda_stream_ptr):

@@ -513,7 +513,7 @@ int vct_destroy(vct_handle c) {
   cudaFree(c->mask_prev[0]); cudaFree(c->mask_prev[1]); cudaFree(c->d_push_list); cudaFree(c->d_push_count);
   cudaFree(c->d_voxrec); cudaFree(c->d_depth); cudaFree(c->d_frags); cudaFree(c->d_items); cudaFree(c->d_counters);
   cudaFree(c->d_vis2[0]); cudaFree(c->d_vis2[1]); cudaFree(c->d_frame);
-  cudaFree(c->d_probe_buf);
+  cudaFree(c->d_stage);
   for (int k = 0; k < 2; ++k) if (c->slot_read_done[k]) cudaEventDestroy(c->slot_read_done[k]);
   if (c->stream_vox) { cudaStreamDestroy(c->stream_vox); cudaEventDestroy(c->ev_vox_done); cudaEventDestroy(c->ev_vtx_done); }
   for (int k = 0; k < 3; ++k) { cudaFree(c->d_frame2[k]); if (c->ev_rendered[k]) cudaEventDestroy(c->ev_rendered[k]); if (c->ev_copied[k]) cudaEventDestroy(c->ev_copied[k]); }
@@ -1272,9 +1272,12 @@ int vct_fragment_count(vct_handle c, uint64_t* n) {
 }
 int vct_debug_counter(vct_handle c, int which, uint64_t* n) {   /* 0 = work items of the last raster pass */
   NEED(c);
-  if (which == 1 || which == 2) {       /* texels the last voxel view visited, textureLod calls of the last probe bake */
+  if (which >= 1 && which <= 3) {   /* texels the last voxel view visited, textureLod calls of the last probe bake,
+                                       texels the last ray cast visited */
     unsigned long long parts[64 * 4];
-    int rc = read_counter(c, which == 1 ? c->d_counters->view_steps : c->d_counters->probe_steps, parts, sizeof(parts));
+    const unsigned long long* d = which == 1 ? c->d_counters->view_steps : which == 2 ? c->d_counters->probe_steps
+                                                                                      : c->d_counters->ray_steps;
+    int rc = read_counter(c, d, parts, sizeof(parts));
     unsigned long long s = 0;
     for (int k = 0; k < 64; ++k) s += parts[k * 4];
     if (n) *n = s;
@@ -1301,6 +1304,20 @@ int vct_trace_cones(vct_handle c, size_t n, const float* starts, const float* di
   return trace_cones(c, n, starts, dirs, tans, out, steps);
 }
 
+// The device staging buffer of the host forms of vct_bake_probes and vct_cast_rays: at least `bytes`, grown on demand.
+// The previous host-form call has completed (each ends in a stream synchronise), so its contents are free.
+static int staging(vct_context* c, size_t bytes, unsigned char** p) {
+  if (c->stage_bytes < bytes) {
+    cudaFree(c->d_stage);
+    c->d_stage = nullptr; c->stage_bytes = 0;
+    VCT_CUDA(c, cudaMalloc(&c->d_stage, bytes));
+    c->stage_bytes = bytes;
+  }
+  *p = c->d_stage;
+  return VCT_OK;
+}
+static size_t up256(size_t b) { return (b + 255) & ~(size_t)255; }
+
 int vct_bake_probes(vct_handle c, size_t n, const float* xyz, float* out, uint32_t* steps, int on_device) {
   NEED(c);
   if (!n) return VCT_OK;
@@ -1310,19 +1327,12 @@ int vct_bake_probes(vct_handle c, size_t n, const float* xyz, float* out, uint32
   if (!c->grid[c->cur].mips_current)   // every cone reads every level
     return set_error(c, VCT_ERR_STATE, "vct_bake_probes: the mip levels are stale (call vct_build_mips after vct_upload_grid_level0)");
   if (on_device) return launch_probes(c, n, xyz, out, steps);
-  // host arrays: staged through one device buffer kept on the context (the previous host-form bake has completed)
-  auto up = [](size_t b) { return (b + 255) & ~(size_t)255; };
   const size_t b_xyz = n * 12, b_out = n * 96, b_steps = steps ? n * 24 : 0;
-  const size_t need = up(b_xyz) + up(b_out) + b_steps;
-  if (c->probe_buf_bytes < need) {
-    cudaFree(c->d_probe_buf);
-    c->d_probe_buf = nullptr; c->probe_buf_bytes = 0;
-    VCT_CUDA(c, cudaMalloc(&c->d_probe_buf, need));
-    c->probe_buf_bytes = need;
-  }
-  float* d_xyz = (float*)c->d_probe_buf;
-  float* d_out = (float*)(c->d_probe_buf + up(b_xyz));
-  uint32_t* d_steps = steps ? (uint32_t*)(c->d_probe_buf + up(b_xyz) + up(b_out)) : nullptr;
+  unsigned char* buf;
+  rc = staging(c, up256(b_xyz) + up256(b_out) + b_steps, &buf); if (rc) return rc;
+  float* d_xyz = (float*)buf;
+  float* d_out = (float*)(buf + up256(b_xyz));
+  uint32_t* d_steps = steps ? (uint32_t*)(buf + up256(b_xyz) + up256(b_out)) : nullptr;
   VCT_CUDA(c, cudaMemcpyAsync(d_xyz, xyz, b_xyz, cudaMemcpyHostToDevice, c->stream));
   rc = launch_probes(c, n, d_xyz, d_out, d_steps);
   cudaError_t e = cudaSuccess;
@@ -1331,6 +1341,44 @@ int vct_bake_probes(vct_handle c, size_t n, const float* xyz, float* out, uint32
   cudaError_t es = cudaStreamSynchronize(c->stream);   // the staging buffer is free again when this returns
   if (rc) return rc;
   return check_cuda(c, e != cudaSuccess ? e : es, "vct_bake_probes");
+}
+
+int vct_cast_rays(vct_handle c, int level, size_t n, const float* segments, uint32_t* voxel, float* t, uint8_t* face,
+                  uint8_t* rgba, uint32_t* steps, int on_device) {
+  NEED(c);
+  if (!n) return VCT_OK;
+  if (level < 0 || level >= c->P.levels) return set_error(c, VCT_ERR_INVALID, "vct_cast_rays: level outside [0, levels)");
+  if (!segments || !voxel) return set_error(c, VCT_ERR_INVALID, "vct_cast_rays: null argument");
+  if (n > SIZE_MAX / 64) return set_error(c, VCT_ERR_INVALID, "vct_cast_rays: n too large");
+  if (on_device && ((uintptr_t)rgba & 3u)) return set_error(c, VCT_ERR_INVALID, "vct_cast_rays: rgba is not 4-byte aligned");
+  int rc = ensure_grid(c); if (rc) return rc;
+  if (level > 0 && !c->grid[c->cur].mips_current)
+    return set_error(c, VCT_ERR_STATE, "vct_cast_rays: the mip levels are stale (call vct_build_mips after vct_upload_grid_level0)");
+  if (on_device) return launch_cast_rays(c, level, n, segments, voxel, t, face, rgba, steps);
+  // host arrays: one region per array in the staging buffer, each 256-byte aligned
+  const size_t b_seg = n * 24, b_voxel = n * 4, b_t = t ? n * 4 : 0, b_face = face ? n : 0, b_rgba = rgba ? n * 4 : 0,
+               b_steps = steps ? n * 4 : 0;
+  unsigned char* buf;
+  rc = staging(c, up256(b_seg) + up256(b_voxel) + up256(b_t) + up256(b_face) + up256(b_rgba) + b_steps, &buf);
+  if (rc) return rc;
+  unsigned char* p = buf;
+  auto take = [&p](size_t b) { unsigned char* q = b ? p : nullptr; p += up256(b); return q; };
+  float* d_seg = (float*)take(b_seg);
+  uint32_t* d_voxel = (uint32_t*)take(b_voxel);
+  float* d_t = (float*)take(b_t);
+  uint8_t* d_face = take(b_face);
+  uint8_t* d_rgba = take(b_rgba);
+  uint32_t* d_steps = (uint32_t*)take(b_steps);
+  VCT_CUDA(c, cudaMemcpyAsync(d_seg, segments, b_seg, cudaMemcpyHostToDevice, c->stream));
+  rc = launch_cast_rays(c, level, n, d_seg, d_voxel, d_t, d_face, d_rgba, d_steps);
+  cudaError_t e = cudaSuccess;
+  const struct { void* host; const void* dev; size_t bytes; } back[] = {
+      {voxel, d_voxel, b_voxel}, {t, d_t, b_t}, {face, d_face, b_face}, {rgba, d_rgba, b_rgba}, {steps, d_steps, b_steps}};
+  for (const auto& b : back)
+    if (!rc && b.host && e == cudaSuccess) e = cudaMemcpyAsync(b.host, b.dev, b.bytes, cudaMemcpyDeviceToHost, c->stream);
+  cudaError_t es = cudaStreamSynchronize(c->stream);   // the staging buffer is free again when this returns
+  if (rc) return rc;
+  return check_cuda(c, e != cudaSuccess ? e : es, "vct_cast_rays");
 }
 
 // ---- execution control

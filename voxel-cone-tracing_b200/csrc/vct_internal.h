@@ -75,6 +75,8 @@ struct Counters {
   unsigned long long view_steps[64 * 4];
   // textureLod calls of the last probe bake (vct_debug_counter 2), partial counters as above, appended last likewise
   unsigned long long probe_steps[64 * 4];
+  // texels visited by the last ray cast (vct_debug_counter 3), partial counters as above, appended last likewise
+  unsigned long long ray_steps[64 * 4];
 };
 
 // Per-vertex transform cache written once per frame by vertex_pass -- the vertex-shader stage of the three
@@ -191,8 +193,8 @@ struct vct_context {
   cudaStream_t copy_stream = nullptr; cudaEvent_t ev_rendered[3]{}, ev_copied[3]{}; bool in_flight[3] = {false, false, false};
   unsigned frame_seq = 0, frame_oldest = 0;
   uint8_t* h_frame_pinned = nullptr; size_t h_frame_bytes = 0;
-  // device staging of vct_bake_probes' host form (probes, results, steps), grown on demand and kept
-  unsigned char* d_probe_buf = nullptr; size_t probe_buf_bytes = 0;
+  // device staging of the host forms of vct_bake_probes and vct_cast_rays (inputs and outputs), grown on demand and kept
+  unsigned char* d_stage = nullptr; size_t stage_bytes = 0;
 
   // timing
   // pass events, VCT_EVENT_GENS generations deep: every frame call (vct_frame, vct_frame_shared_begin) moves to the
@@ -251,6 +253,8 @@ int launch_cone(vct_context* c);
 int launch_reinject(vct_context* c);
 int launch_voxel_view(vct_context* c, int level, const float inv_vp[16], uint32_t* d_voxel);   // vct_view.cu
 int launch_probes(vct_context* c, size_t n, const float* xyz, float* out, uint32_t* steps);     // device pointers
+int launch_cast_rays(vct_context* c, int level, size_t n, const float* seg, uint32_t* voxel, float* t, uint8_t* face,
+                     uint8_t* rgba, uint32_t* steps);                                           // vct_view.cu, device pointers
 int check_overflow(vct_context* c);
 int comm_barrier(vct_context* c, int channel, cudaStream_t stream);   // device-side cross-rank barrier, in stream order
 int comm_check(vct_context* c);                                        // barrier time-outs -> VCT_ERR_STATE

@@ -167,6 +167,14 @@ struct Voxel_Cone_Tracing {
     check(vct_bake_probes(device, n, xyz, out, steps, 0));
   }
 
+  // ray casts (no reference counterpart): the first occupied texel of mip `level` of the current pyramid along n
+  // world-space segments (segments: n*6, a.xyz b.xyz); voxel: n texel indices (0xFFFFFFFF = miss); t, face (1..6 =
+  // +X, -X, +Y, -Y, +Z, -Z), rgba (n*4) and steps may be NULL
+  void CastRays(int level, const float* segments, size_t n, uint32_t* voxel, float* t = nullptr, uint8_t* face = nullptr,
+                uint8_t* rgba = nullptr, uint32_t* steps = nullptr) {
+    check(vct_cast_rays(device, level, n, segments, voxel, t, face, rgba, steps, 0));
+  }
+
   // the uniform block of Render() (Voxel_Cone_Tracing.h:161-187), separated so that a sharded frame can set it too
   void SetRenderUniforms() {
     mat4 vMat = camera.GetViewMatrix();

@@ -4,8 +4,9 @@
 //   facade_demo [dump_dir]   with a directory: also writes the flattened scene (verts.f32, idx.u32, trimat.u16), the
 //   uniforms of every frame (uniforms_<f>.f32: ModelView, Projection, DepthMVP, ProjX, ProjY, ProjZ, camera) and the
 //   frames (frame_<f>.rgba), voxel views of mip level 1 (voxels_<f>.rgba) and, after the frames, the irradiance probes
-//   of the cell centres of an 8x8x8 lattice over the grid (probe_xyz.f32, probes.f32), so that a test can replay the
-//   same inputs through another binding and compare bytes.
+//   of the cell centres of an 8x8x8 lattice over the grid (probe_xyz.f32, probes.f32) and the level-0 ray casts of a
+//   fan of 16x16 segments from the grid's centre to the cell centres of its -Z face (rays_seg.f32, rays_voxel.u32,
+//   rays_t.f32), so that a test can replay the same inputs through another binding and compare bytes.
 //   facade_demo <dump_dir> sharded [second_device]   also renders the views as sharded frames over two ranks.
 #include <cstdio>
 #include <cstdlib>
@@ -99,6 +100,20 @@ int main(int argc, char** argv) {
       voxel_cone_tracing.BakeProbes(xyz.data(), (size_t)k * k * k, probes.data());
       dump(dir + "probe_xyz.f32", xyz.data(), xyz.size() * sizeof(float));
       dump(dir + "probes.f32", probes.data(), probes.size() * sizeof(float));
+      const int r = 16;
+      const float rcell = G / (float)r;
+      std::vector<float> seg;
+      for (int y = 0; y < r; ++y)
+        for (int x = 0; x < r; ++x) {
+          const float b[3] = {((float)x + 0.5f) * rcell - 0.5f * G, ((float)y + 0.5f) * rcell - 0.5f * G, -0.5f * G};
+          seg.insert(seg.end(), {0.0f, 0.0f, 0.0f, b[0], b[1], b[2]});
+        }
+      std::vector<uint32_t> ray_voxel((size_t)r * r);
+      std::vector<float> ray_t((size_t)r * r);
+      voxel_cone_tracing.CastRays(0, seg.data(), (size_t)r * r, ray_voxel.data(), ray_t.data());
+      dump(dir + "rays_seg.f32", seg.data(), seg.size() * sizeof(float));
+      dump(dir + "rays_voxel.u32", ray_voxel.data(), ray_voxel.size() * sizeof(uint32_t));
+      dump(dir + "rays_t.f32", ray_t.data(), ray_t.size() * sizeof(float));
     }
     // The same three views as ONE sharded frame stream over two ranks (two GPUs if the machine has them, else two
     // handles on GPU 0): the frames must equal the single-GPU ones byte for byte.

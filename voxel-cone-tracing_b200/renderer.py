@@ -164,6 +164,13 @@ class Voxel_Cone_Tracing:
         self._set_render_uniforms()
         return self.ctx.bake_probes(xyz)
 
+    def CastRays(self, level, a, b):
+        """Ray casts (no reference counterpart): the first occupied texel of mip `level` of the current pyramid along each
+        world-space segment a[i] -> b[i] ((n, 3) each).  Returns (voxel, t, face, rgba, steps) as Context.cast_rays."""
+        self._set_render_uniforms()   # VoxelGridWorldSize; the camera uniforms it also sets have no effect on a cast
+        seg = np.concatenate([np.asarray(a, np.float32).reshape(-1, 3), np.asarray(b, np.float32).reshape(-1, 3)], 1)
+        return self.ctx.cast_rays(level, seg)
+
     def Frame(self, out=None):
         """DrawVoxelTexture + Render in one call (what 'full frames/s' times)."""
         self._set_render_uniforms()
