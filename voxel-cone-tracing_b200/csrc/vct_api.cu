@@ -21,9 +21,6 @@ int check_cuda(vct_context* c, cudaError_t e, const char* what) {
 }
 
 int readback_accum(vct_context* c, uint32_t* counts, uint32_t* sums);
-int sample_voxels(vct_context* c, size_t n, const float* pos, const float* lod, float* out);
-int trace_cones(vct_context* c, size_t n, const float* starts, const float* dirs, const float* tans, float* out,
-                uint32_t* steps);
 
 // ------------------------------------------------------------------------------------------ helpers
 static int ilog2(int v) { int l = 0; while ((1 << l) < v) ++l; return l; }
@@ -419,6 +416,52 @@ int begin_voxel_slot(vct_context* c) {
   return VCT_OK;
 }
 
+// ---- queries on the pyramid
+// The pyramid of a query that reads levels 0..top: allocated, and its levels above 0 built from level 0 if it reads any.
+static int need_pyramid(vct_context* c, const char* what, int top) {
+  int rc = ensure_grid(c); if (rc) return rc;
+  if (top > 0 && !c->grid[c->cur].mips_current)
+    return set_error(c, VCT_ERR_STATE, std::string(what) + ": the mip levels are stale (call vct_build_mips after vct_upload_grid_level0)");
+  return VCT_OK;
+}
+
+// One host array of a call: `in` is copied to the device before the launch, `out` back after it.  Neither: the array
+// is absent.
+struct HostArray { const void* in; void* out; size_t bytes; };
+
+// The host form of a device call.  Lays out the arrays in c->d_stage (grown on demand), each present one in its own
+// 256-byte-aligned region, copies the inputs there on c->stream, runs launch(d) with d[k] the device pointer of a[k]
+// (NULL for an absent array), copies the outputs back and synchronises c->stream once, error paths included, so that
+// the buffer is free for the next call when this returns.  Returns the launch's own error code if it failed, else the
+// first copy error, else the synchronise's.
+template <size_t N, class Launch>
+static int host_round_trip(vct_context* c, const char* what, const HostArray (&a)[N], Launch launch) {
+  auto up256 = [](size_t b) { return (b + 255) & ~(size_t)255; };
+  size_t bytes = 0;
+  for (const HostArray& x : a) if (x.in || x.out) bytes += up256(x.bytes);
+  if (c->stage_bytes < bytes) {
+    cudaFree(c->d_stage);
+    c->d_stage = nullptr; c->stage_bytes = 0;
+    VCT_CUDA(c, cudaMalloc(&c->d_stage, bytes));
+    c->stage_bytes = bytes;
+  }
+  void* d[N];
+  unsigned char* p = c->d_stage;
+  for (size_t k = 0; k < N; ++k) {
+    d[k] = a[k].in || a[k].out ? p : nullptr;
+    if (d[k]) p += up256(a[k].bytes);
+  }
+  cudaError_t e = cudaSuccess;
+  for (size_t k = 0; k < N; ++k)
+    if (a[k].in && e == cudaSuccess) e = cudaMemcpyAsync(d[k], a[k].in, a[k].bytes, cudaMemcpyHostToDevice, c->stream);
+  const int rc = e == cudaSuccess ? launch(d) : VCT_OK;
+  for (size_t k = 0; k < N; ++k)
+    if (!rc && a[k].out && e == cudaSuccess) e = cudaMemcpyAsync(a[k].out, d[k], a[k].bytes, cudaMemcpyDeviceToHost, c->stream);
+  const cudaError_t es = cudaStreamSynchronize(c->stream);
+  if (rc) return rc;
+  return check_cuda(c, e != cudaSuccess ? e : es, what);
+}
+
 // ------------------------------------------------------------------------------------------ tex bench
 __global__ void fill_level_random(cudaSurfaceObject_t s, int n, unsigned seed, int f16) {
   int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y * blockDim.y + threadIdx.y, z = blockIdx.z;
@@ -726,20 +769,17 @@ __global__ void scatter_positions(const float* __restrict__ xyz, float* __restri
 int vct_update_positions(vct_handle c, const float* xyz, size_t nv, int on_device) {
   NEED(c);
   if (!xyz || nv != c->nv) return set_error(c, VCT_ERR_INVALID, "vct_update_positions: vertex count mismatch");
-  const float* src = xyz;
-  float* tmp = nullptr;
-  if (!on_device) {
-    VCT_CUDA(c, cudaMalloc(&tmp, nv * 12));
-    VCT_CUDA(c, cudaMemcpyAsync(tmp, xyz, nv * 12, cudaMemcpyHostToDevice, c->stream));
-    src = tmp;
-  }
-  scatter_positions<<<(unsigned)((nv + 255) / 256), 256, 0, c->stream>>>(src, c->d_verts, nv);
-  c->launches += 1;
-  if (tmp) { cudaStreamSynchronize(c->stream); cudaFree(tmp); }
-  c->depth_valid = false;
-  c->vcache_valid[0] = c->vcache_valid[1] = false;
-  c->scene_epoch++;
-  return check_cuda(c, cudaGetLastError(), "scatter_positions");
+  auto scatter = [&](const float* src) {
+    scatter_positions<<<(unsigned)((nv + 255) / 256), 256, 0, c->stream>>>(src, c->d_verts, nv);
+    c->launches += 1;
+    c->depth_valid = false;
+    c->vcache_valid[0] = c->vcache_valid[1] = false;
+    c->scene_epoch++;
+    return check_cuda(c, cudaGetLastError(), "scatter_positions");
+  };
+  if (on_device) return scatter(xyz);
+  return host_round_trip(c, "vct_update_positions", {{xyz, nullptr, nv * 12}},
+                         [&](void* const* d) { return scatter((const float*)d[0]); });
 }
 
 // ---- passes
@@ -987,24 +1027,19 @@ static void voxel_view_matrix(const Params& P, float* inv_vp) {
 
 int vct_render_voxels(vct_handle c, int level, uint8_t* host_rgba, uint32_t* host_voxel) {
   NEED(c);
-  int rc = ensure_grid(c); if (rc) return rc;
   if (level < 0 || level >= c->P.levels) return set_error(c, VCT_ERR_INVALID, "vct_render_voxels: level outside [0, levels)");
-  if (level > 0 && !c->grid[c->cur].mips_current)
-    return set_error(c, VCT_ERR_STATE, "vct_render_voxels: the mip levels are stale (call vct_build_mips after vct_upload_grid_level0)");
+  int rc = need_pyramid(c, "vct_render_voxels", level); if (rc) return rc;
   rc = ensure_frame(c); if (rc) return rc;
   float inv_vp[16];
   voxel_view_matrix(c->P, inv_vp);
+  if (!host_rgba && !host_voxel) return launch_voxel_view(c, level, inv_vp, nullptr);
   const size_t n = (size_t)c->P.W * c->P.H;
-  uint32_t* d_voxel = nullptr;
-  if (host_voxel) VCT_CUDA(c, cudaMalloc(&d_voxel, n * 4));
-  rc = launch_voxel_view(c, level, inv_vp, d_voxel);
-  cudaError_t e = cudaSuccess;
-  if (!rc && host_rgba) e = cudaMemcpyAsync(host_rgba, c->d_frame, n * 4, cudaMemcpyDeviceToHost, c->stream);
-  if (!rc && host_voxel && e == cudaSuccess) e = cudaMemcpyAsync(host_voxel, d_voxel, n * 4, cudaMemcpyDeviceToHost, c->stream);
-  if (!rc && (host_rgba || host_voxel) && e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  if (d_voxel) { if (rc || e != cudaSuccess) cudaStreamSynchronize(c->stream); cudaFree(d_voxel); }
-  if (rc) return rc;
-  return check_cuda(c, e, "vct_render_voxels");
+  return host_round_trip(c, "vct_render_voxels", {{nullptr, host_voxel, n * 4}}, [&](void* const* d) {
+    const int r = launch_voxel_view(c, level, inv_vp, (uint32_t*)d[0]);
+    if (r || !host_rgba) return r;
+    // the view itself is in the frame buffer
+    return check_cuda(c, cudaMemcpyAsync(host_rgba, c->d_frame, n * 4, cudaMemcpyDeviceToHost, c->stream), "vct_render_voxels");
+  });
 }
 
 static int ensure_overlap(vct_context* c) {
@@ -1222,14 +1257,11 @@ int vct_readback_visibility(vct_handle c, uint32_t* tri) {
   NEED(c);
   if (!c->d_vis2[c->cur] || !tri) return set_error(c, VCT_ERR_STATE, "no frame rendered");
   const size_t n = (size_t)c->P.W * c->P.H;
-  uint32_t* d = nullptr;
-  VCT_CUDA(c, cudaMalloc(&d, n * 4));
-  vis_to_tri<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->d_vis2[c->cur], d, n);
-  c->launches += 1;
-  cudaError_t e = cudaMemcpyAsync(tri, d, n * 4, cudaMemcpyDeviceToHost, c->stream);
-  if (e == cudaSuccess) e = cudaStreamSynchronize(c->stream);
-  cudaFree(d);
-  return check_cuda(c, e, "vct_readback_visibility");
+  return host_round_trip(c, "vct_readback_visibility", {{nullptr, tri, n * 4}}, [&](void* const* d) {
+    vis_to_tri<<<(unsigned)((n + 255) / 256), 256, 0, c->stream>>>(c->d_vis2[c->cur], (uint32_t*)d[0], n);
+    c->launches += 1;
+    return check_cuda(c, cudaGetLastError(), "vis_to_tri");
+  });
 }
 
 int vct_readback_frame(vct_handle c, uint8_t* rgba) {
@@ -1254,15 +1286,15 @@ static int read_counter(vct_context* c, const void* dptr, void* out, size_t byte
   VCT_CUDA(c, cudaMemcpyAsync(out, dptr, bytes, cudaMemcpyDeviceToHost, c->stream));
   return check_cuda(c, cudaStreamSynchronize(c->stream), "sync");
 }
-int vct_cone_samples(vct_handle c, uint64_t* n) {
-  NEED(c);
+static int read_steps(vct_context* c, StepCounter k, uint64_t* n) {
   unsigned long long parts[64 * 4];
-  int rc = read_counter(c, c->d_counters->cone_samples, parts, sizeof(parts));
+  int rc = read_counter(c, c->d_counters->steps[k], parts, sizeof(parts));
   unsigned long long v = 0;
-  for (int k = 0; k < 64; ++k) v += parts[k * 4];
+  for (int s = 0; s < 64; ++s) v += parts[s * 4];
   if (n) *n = v;
   return rc;
 }
+int vct_cone_samples(vct_handle c, uint64_t* n) { NEED(c); return read_steps(c, STEPS_CONE, n); }
 int vct_fragment_count(vct_handle c, uint64_t* n) {
   NEED(c);
   unsigned int v = 0;
@@ -1272,17 +1304,7 @@ int vct_fragment_count(vct_handle c, uint64_t* n) {
 }
 int vct_debug_counter(vct_handle c, int which, uint64_t* n) {   /* 0 = work items of the last raster pass */
   NEED(c);
-  if (which >= 1 && which <= 3) {   /* texels the last voxel view visited, textureLod calls of the last probe bake,
-                                       texels the last ray cast visited */
-    unsigned long long parts[64 * 4];
-    const unsigned long long* d = which == 1 ? c->d_counters->view_steps : which == 2 ? c->d_counters->probe_steps
-                                                                                      : c->d_counters->ray_steps;
-    int rc = read_counter(c, d, parts, sizeof(parts));
-    unsigned long long s = 0;
-    for (int k = 0; k < 64; ++k) s += parts[k * 4];
-    if (n) *n = s;
-    return rc;
-  }
+  if (which >= STEPS_VIEW && which <= STEPS_RAYS) return read_steps(c, (StepCounter)which, n);
   unsigned int v = 0;
   int rc = read_counter(c, which == 0 ? (const void*)&c->d_counters->n_items : (const void*)&c->d_counters->overflow, &v, 4);
   if (n) *n = v;
@@ -1301,46 +1323,26 @@ int vct_trace_cones(vct_handle c, size_t n, const float* starts, const float* di
                     uint32_t* steps) {
   NEED(c);
   if (n && (!starts || !dirs || !tans || !out)) return set_error(c, VCT_ERR_INVALID, "vct_trace_cones: null argument");
-  return trace_cones(c, n, starts, dirs, tans, out, steps);
+  int rc = ensure_grid(c); if (rc) return rc;
+  if (!n) return VCT_OK;
+  return host_round_trip(c, "vct_trace_cones",
+                         {{starts, nullptr, n * 12}, {dirs, nullptr, n * 12}, {tans, nullptr, n * 4}, {nullptr, out, n * 16},
+                          {nullptr, steps, n * 4}},
+                         [&](void* const* d) {
+                           return launch_trace_cones(c, n, (const float*)d[0], (const float*)d[1], (const float*)d[2],
+                                                     (float*)d[3], (uint32_t*)d[4]);
+                         });
 }
-
-// The device staging buffer of the host forms of vct_bake_probes and vct_cast_rays: at least `bytes`, grown on demand.
-// The previous host-form call has completed (each ends in a stream synchronise), so its contents are free.
-static int staging(vct_context* c, size_t bytes, unsigned char** p) {
-  if (c->stage_bytes < bytes) {
-    cudaFree(c->d_stage);
-    c->d_stage = nullptr; c->stage_bytes = 0;
-    VCT_CUDA(c, cudaMalloc(&c->d_stage, bytes));
-    c->stage_bytes = bytes;
-  }
-  *p = c->d_stage;
-  return VCT_OK;
-}
-static size_t up256(size_t b) { return (b + 255) & ~(size_t)255; }
 
 int vct_bake_probes(vct_handle c, size_t n, const float* xyz, float* out, uint32_t* steps, int on_device) {
   NEED(c);
   if (!n) return VCT_OK;
   if (!xyz || !out) return set_error(c, VCT_ERR_INVALID, "vct_bake_probes: null argument");
   if (n > SIZE_MAX / 256) return set_error(c, VCT_ERR_INVALID, "vct_bake_probes: n too large");
-  int rc = ensure_grid(c); if (rc) return rc;
-  if (!c->grid[c->cur].mips_current)   // every cone reads every level
-    return set_error(c, VCT_ERR_STATE, "vct_bake_probes: the mip levels are stale (call vct_build_mips after vct_upload_grid_level0)");
+  int rc = need_pyramid(c, "vct_bake_probes", c->P.levels - 1); if (rc) return rc;   // every cone reads every level
   if (on_device) return launch_probes(c, n, xyz, out, steps);
-  const size_t b_xyz = n * 12, b_out = n * 96, b_steps = steps ? n * 24 : 0;
-  unsigned char* buf;
-  rc = staging(c, up256(b_xyz) + up256(b_out) + b_steps, &buf); if (rc) return rc;
-  float* d_xyz = (float*)buf;
-  float* d_out = (float*)(buf + up256(b_xyz));
-  uint32_t* d_steps = steps ? (uint32_t*)(buf + up256(b_xyz) + up256(b_out)) : nullptr;
-  VCT_CUDA(c, cudaMemcpyAsync(d_xyz, xyz, b_xyz, cudaMemcpyHostToDevice, c->stream));
-  rc = launch_probes(c, n, d_xyz, d_out, d_steps);
-  cudaError_t e = cudaSuccess;
-  if (!rc) e = cudaMemcpyAsync(out, d_out, b_out, cudaMemcpyDeviceToHost, c->stream);
-  if (!rc && steps && e == cudaSuccess) e = cudaMemcpyAsync(steps, d_steps, b_steps, cudaMemcpyDeviceToHost, c->stream);
-  cudaError_t es = cudaStreamSynchronize(c->stream);   // the staging buffer is free again when this returns
-  if (rc) return rc;
-  return check_cuda(c, e != cudaSuccess ? e : es, "vct_bake_probes");
+  return host_round_trip(c, "vct_bake_probes", {{xyz, nullptr, n * 12}, {nullptr, out, n * 96}, {nullptr, steps, n * 24}},
+                         [&](void* const* d) { return launch_probes(c, n, (const float*)d[0], (float*)d[1], (uint32_t*)d[2]); });
 }
 
 int vct_cast_rays(vct_handle c, int level, size_t n, const float* segments, uint32_t* voxel, float* t, uint8_t* face,
@@ -1351,41 +1353,27 @@ int vct_cast_rays(vct_handle c, int level, size_t n, const float* segments, uint
   if (!segments || !voxel) return set_error(c, VCT_ERR_INVALID, "vct_cast_rays: null argument");
   if (n > SIZE_MAX / 64) return set_error(c, VCT_ERR_INVALID, "vct_cast_rays: n too large");
   if (on_device && ((uintptr_t)rgba & 3u)) return set_error(c, VCT_ERR_INVALID, "vct_cast_rays: rgba is not 4-byte aligned");
-  int rc = ensure_grid(c); if (rc) return rc;
-  if (level > 0 && !c->grid[c->cur].mips_current)
-    return set_error(c, VCT_ERR_STATE, "vct_cast_rays: the mip levels are stale (call vct_build_mips after vct_upload_grid_level0)");
+  int rc = need_pyramid(c, "vct_cast_rays", level); if (rc) return rc;
   if (on_device) return launch_cast_rays(c, level, n, segments, voxel, t, face, rgba, steps);
-  // host arrays: one region per array in the staging buffer, each 256-byte aligned
-  const size_t b_seg = n * 24, b_voxel = n * 4, b_t = t ? n * 4 : 0, b_face = face ? n : 0, b_rgba = rgba ? n * 4 : 0,
-               b_steps = steps ? n * 4 : 0;
-  unsigned char* buf;
-  rc = staging(c, up256(b_seg) + up256(b_voxel) + up256(b_t) + up256(b_face) + up256(b_rgba) + b_steps, &buf);
-  if (rc) return rc;
-  unsigned char* p = buf;
-  auto take = [&p](size_t b) { unsigned char* q = b ? p : nullptr; p += up256(b); return q; };
-  float* d_seg = (float*)take(b_seg);
-  uint32_t* d_voxel = (uint32_t*)take(b_voxel);
-  float* d_t = (float*)take(b_t);
-  uint8_t* d_face = take(b_face);
-  uint8_t* d_rgba = take(b_rgba);
-  uint32_t* d_steps = (uint32_t*)take(b_steps);
-  VCT_CUDA(c, cudaMemcpyAsync(d_seg, segments, b_seg, cudaMemcpyHostToDevice, c->stream));
-  rc = launch_cast_rays(c, level, n, d_seg, d_voxel, d_t, d_face, d_rgba, d_steps);
-  cudaError_t e = cudaSuccess;
-  const struct { void* host; const void* dev; size_t bytes; } back[] = {
-      {voxel, d_voxel, b_voxel}, {t, d_t, b_t}, {face, d_face, b_face}, {rgba, d_rgba, b_rgba}, {steps, d_steps, b_steps}};
-  for (const auto& b : back)
-    if (!rc && b.host && e == cudaSuccess) e = cudaMemcpyAsync(b.host, b.dev, b.bytes, cudaMemcpyDeviceToHost, c->stream);
-  cudaError_t es = cudaStreamSynchronize(c->stream);   // the staging buffer is free again when this returns
-  if (rc) return rc;
-  return check_cuda(c, e != cudaSuccess ? e : es, "vct_cast_rays");
+  return host_round_trip(c, "vct_cast_rays",
+                         {{segments, nullptr, n * 24}, {nullptr, voxel, n * 4}, {nullptr, t, n * 4}, {nullptr, face, n},
+                          {nullptr, rgba, n * 4}, {nullptr, steps, n * 4}},
+                         [&](void* const* d) {
+                           return launch_cast_rays(c, level, n, (const float*)d[0], (uint32_t*)d[1], (float*)d[2],
+                                                   (uint8_t*)d[3], (uint8_t*)d[4], (uint32_t*)d[5]);
+                         });
 }
 
 // ---- execution control
 int vct_sample_voxels(vct_handle c, size_t n, const float* pos, const float* lod, float* out) {
   NEED(c);
   if (n && (!pos || !lod || !out)) return set_error(c, VCT_ERR_INVALID, "vct_sample_voxels: null argument");
-  return sample_voxels(c, n, pos, lod, out);
+  int rc = ensure_grid(c); if (rc) return rc;
+  if (!n) return VCT_OK;
+  return host_round_trip(c, "vct_sample_voxels", {{pos, nullptr, n * 12}, {lod, nullptr, n * 4}, {nullptr, out, n * 16}},
+                         [&](void* const* d) {
+                           return launch_sample_voxels(c, n, (const float*)d[0], (const float*)d[1], (float*)d[2]);
+                         });
 }
 
 int vct_set_stream(vct_handle c, void* s) {

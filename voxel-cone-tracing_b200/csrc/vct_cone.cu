@@ -523,10 +523,7 @@ __global__ void __launch_bounds__(BT, MINB) cone_trace(Params P, VertexCache vc,
     }
     frame[(size_t)j * P.W + i] = out;
   }
-  // executed textureLod calls (Gcone-samples/s numerator): one atomic per warp
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) samples += __shfl_xor_sync(0xffffffffu, samples, d);
-  if (lane == 0 && samples) atomicAdd(&ctr->cone_samples[((blockIdx.x + blockIdx.y * 7u) & 63u) * 4], (unsigned long long)samples);
+  count_steps(ctr, STEPS_CONE, lane, samples, [] { return (blockIdx.x + blockIdx.y * 7u) & 63u; });   // Gcone-samples/s numerator
 }
 
 int launch_cone(vct_context* c) {
@@ -535,7 +532,7 @@ int launch_cone(vct_context* c) {
   if (!c->depth_valid) return set_error(c, VCT_ERR_STATE, "vct_render: call vct_draw_depth first (shadow map missing)");
   rc = ensure_vertex_cache(c); if (rc) return rc;
   PassTimer timer(c, VCT_PASS_CONE);
-  VCT_CUDA(c, cudaMemsetAsync(c->d_counters->cone_samples, 0, sizeof(c->d_counters->cone_samples), c->stream));
+  VCT_CUDA(c, reset_steps(c, STEPS_CONE));
   int y0 = c->P.row_begin, y1 = (c->P.row_end > 0 && c->P.row_end < c->P.H) ? c->P.row_end : c->P.H;
   const bool strips = c->P.row_il > 1;
   int own_groups = 0;                              // interleaved strips: how many groups of 8 rows this context owns
@@ -654,23 +651,12 @@ __global__ void trace_cones_kernel(Params P, cudaTextureObject_t grid, size_t n,
   if (steps) steps[i] = cnt;
 }
 
-int trace_cones(vct_context* c, size_t n, const float* starts, const float* dirs, const float* tans, float* out,
-                uint32_t* steps) {
-  int rc = ensure_grid(c); if (rc) return rc;
-  if (!n) return VCT_OK;
-  float *d_s = nullptr, *d_d = nullptr, *d_t = nullptr; float4* d_o = nullptr; uint32_t* d_n = nullptr;
-  VCT_CUDA(c, cudaMalloc(&d_s, n * 12)); VCT_CUDA(c, cudaMalloc(&d_d, n * 12)); VCT_CUDA(c, cudaMalloc(&d_t, n * 4));
-  VCT_CUDA(c, cudaMalloc(&d_o, n * 16)); VCT_CUDA(c, cudaMalloc(&d_n, n * 4));
-  cudaMemcpyAsync(d_s, starts, n * 12, cudaMemcpyHostToDevice, c->stream);
-  cudaMemcpyAsync(d_d, dirs, n * 12, cudaMemcpyHostToDevice, c->stream);
-  cudaMemcpyAsync(d_t, tans, n * 4, cudaMemcpyHostToDevice, c->stream);
-  trace_cones_kernel<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->P, c->grid[c->cur].tex, n, d_s, d_d, d_t, d_o, d_n);
+int launch_trace_cones(vct_context* c, size_t n, const float* starts, const float* dirs, const float* tans, float* out,
+                       uint32_t* steps) {
+  trace_cones_kernel<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->P, c->grid[c->cur].tex, n, starts, dirs, tans,
+                                                                         (float4*)out, steps);
   c->launches += 1;
-  cudaMemcpyAsync(out, d_o, n * 16, cudaMemcpyDeviceToHost, c->stream);
-  if (steps) cudaMemcpyAsync(steps, d_n, n * 4, cudaMemcpyDeviceToHost, c->stream);
-  cudaError_t e = cudaStreamSynchronize(c->stream);
-  cudaFree(d_s); cudaFree(d_d); cudaFree(d_t); cudaFree(d_o); cudaFree(d_n);
-  return check_cuda(c, e, "vct_trace_cones");
+  return check_cuda(c, cudaGetLastError(), "trace_cones");
 }
 
 // Irradiance probes (vct_bake_probes, no reference counterpart): the frame's diffuse term (VoxelConeTracing.fs:92,
@@ -718,10 +704,7 @@ __global__ void __launch_bounds__(PROBE_BT) bake_probes_kernel(Params P, ProbeBa
     o[0] = r.x; o[1] = r.y; o[2] = r.z; o[3] = r.w;
     if (steps) steps[p * 6 + face] = cnt;
   }
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) cnt += __shfl_xor_sync(0xffffffffu, cnt, d);
-  if ((threadIdx.x & 31) == 0 && cnt)
-    atomicAdd(&ctr->probe_steps[((blockIdx.x + blockIdx.y * 7u) & 63u) * 4], (unsigned long long)cnt);
+  count_steps(ctr, STEPS_PROBES, threadIdx.x & 31, cnt, [] { return (blockIdx.x + blockIdx.y * 7u) & 63u; });
 }
 
 int launch_probes(vct_context* c, size_t n, const float* xyz, float* out, uint32_t* steps) {
@@ -732,7 +715,7 @@ int launch_probes(vct_context* c, size_t n, const float* xyz, float* out, uint32
   const size_t blocks = (n + PROBE_BT - 1) / PROBE_BT;
   if (blocks > 0x7fffffffu) return set_error(c, VCT_ERR_INVALID, "vct_bake_probes: too many probes for one launch");
   PassTimer timer(c, VCT_PASS_PROBES);
-  VCT_CUDA(c, cudaMemsetAsync(c->d_counters->probe_steps, 0, sizeof(c->d_counters->probe_steps), c->stream));
+  VCT_CUDA(c, reset_steps(c, STEPS_PROBES));
   bake_probes_kernel<<<dim3((unsigned)blocks, 6), PROBE_BT, 0, c->stream>>>(c->P, basis, c->grid[c->cur].tex, n, xyz, out,
                                                                              steps, c->d_counters);
   c->launches += 1;
@@ -749,19 +732,10 @@ __global__ void sample_voxels_kernel(Params P, cudaTextureObject_t grid, size_t 
   out[i] = tex3DLod<float4>(grid, u, v, w, lod[i]);
 }
 
-int sample_voxels(vct_context* c, size_t n, const float* pos, const float* lod, float* out) {
-  int rc = ensure_grid(c); if (rc) return rc;
-  if (!n) return VCT_OK;
-  float *d_p = nullptr, *d_l = nullptr; float4* d_o = nullptr;
-  VCT_CUDA(c, cudaMalloc(&d_p, n * 12)); VCT_CUDA(c, cudaMalloc(&d_l, n * 4)); VCT_CUDA(c, cudaMalloc(&d_o, n * 16));
-  cudaMemcpyAsync(d_p, pos, n * 12, cudaMemcpyHostToDevice, c->stream);
-  cudaMemcpyAsync(d_l, lod, n * 4, cudaMemcpyHostToDevice, c->stream);
-  sample_voxels_kernel<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->P, c->grid[c->cur].tex, n, d_p, d_l, d_o);
+int launch_sample_voxels(vct_context* c, size_t n, const float* pos, const float* lod, float* out) {
+  sample_voxels_kernel<<<(unsigned)((n + 127) / 128), 128, 0, c->stream>>>(c->P, c->grid[c->cur].tex, n, pos, lod, (float4*)out);
   c->launches += 1;
-  cudaMemcpyAsync(out, d_o, n * 16, cudaMemcpyDeviceToHost, c->stream);
-  cudaError_t e = cudaStreamSynchronize(c->stream);
-  cudaFree(d_p); cudaFree(d_l); cudaFree(d_o);
-  return check_cuda(c, e, "vct_sample_voxels");
+  return check_cuda(c, cudaGetLastError(), "sample_voxels");
 }
 
 }  // namespace vct

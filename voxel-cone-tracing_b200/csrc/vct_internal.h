@@ -5,6 +5,7 @@
 #pragma once
 
 #include <cuda_runtime.h>
+#include <stddef.h>
 #include <stdint.h>
 
 #include <string>
@@ -58,6 +59,10 @@ struct TextureEntry {
 
 struct MaterialHost { int d = -1, s = -1, h = -1; float shininess = 20.0f; };
 
+// Kernels that count their work, numbered as vct_debug_counter reads them: executed textureLod calls of cone_trace
+// (vct_cone_samples), texels visited by the voxel view, textureLod calls of the probe bake, texels visited by ray casts
+enum StepCounter { STEPS_CONE, STEPS_VIEW, STEPS_PROBES, STEPS_RAYS, N_STEP_COUNTERS };
+
 // Device counters, one cache line each to keep unrelated atomics apart.
 struct Counters {
   unsigned int n_fragments;   unsigned int pad0[31];
@@ -67,17 +72,13 @@ struct Counters {
   unsigned int n_items, next_item, items_overflow; unsigned int pad1[29];
   unsigned int n_touched;     unsigned int pad2[31];
   unsigned int overflow;      unsigned int pad3[31];   // sticky until read by check_overflow
-  // executed textureLod calls of the last cone_trace: 64 partial counters, one 32-byte sector each (65 K warps adding
-  // into ONE address serialise in a single L2 atomic unit); vct_cone_samples sums them
-  unsigned long long cone_samples[64 * 4];
-  // texels visited by the last voxel view (vct_debug_counter 1), partial counters as above.  Appended last so that no
-  // field the other kernels address moves.
-  unsigned long long view_steps[64 * 4];
-  // textureLod calls of the last probe bake (vct_debug_counter 2), partial counters as above, appended last likewise
-  unsigned long long probe_steps[64 * 4];
-  // texels visited by the last ray cast (vct_debug_counter 3), partial counters as above, appended last likewise
-  unsigned long long ray_steps[64 * 4];
+  // the work of the last launch of each counting kernel (StepCounter) as 64 partial counters, one 32-byte sector each
+  // (65 K warps adding into ONE address serialise in a single L2 atomic unit): count_steps adds, reset_steps clears,
+  // read_steps sums them
+  unsigned long long steps[N_STEP_COUNTERS][64 * 4];
 };
+static_assert(offsetof(Counters, steps) == 512, "the step counters start after the four counter lines");
+static_assert(sizeof(Counters) == 8704, "Counters: four counter lines and four step counters");
 
 // Per-vertex transform cache written once per frame by vertex_pass -- the vertex-shader stage of the three
 // reference programs (Voxelization.vs:15-22, VoxelConeTracing.vs:23-37) evaluated once per vertex, as GL does,
@@ -193,7 +194,8 @@ struct vct_context {
   cudaStream_t copy_stream = nullptr; cudaEvent_t ev_rendered[3]{}, ev_copied[3]{}; bool in_flight[3] = {false, false, false};
   unsigned frame_seq = 0, frame_oldest = 0;
   uint8_t* h_frame_pinned = nullptr; size_t h_frame_bytes = 0;
-  // device staging of the host forms of vct_bake_probes and vct_cast_rays (inputs and outputs), grown on demand and kept
+  // device staging of the calls that run a kernel on host arrays (host_round_trip): their inputs and outputs, grown on
+  // demand and kept.  Each such call ends in a stream synchronise, so the next one finds the buffer free.
   unsigned char* d_stage = nullptr; size_t stage_bytes = 0;
 
   // timing
@@ -252,9 +254,13 @@ int launch_visibility(vct_context* c);
 int launch_cone(vct_context* c);
 int launch_reinject(vct_context* c);
 int launch_voxel_view(vct_context* c, int level, const float inv_vp[16], uint32_t* d_voxel);   // vct_view.cu
-int launch_probes(vct_context* c, size_t n, const float* xyz, float* out, uint32_t* steps);     // device pointers
+// queries on the current pyramid, all pointers on the device
+int launch_trace_cones(vct_context* c, size_t n, const float* starts, const float* dirs, const float* tans, float* out,
+                       uint32_t* steps);
+int launch_sample_voxels(vct_context* c, size_t n, const float* pos, const float* lod, float* out);
+int launch_probes(vct_context* c, size_t n, const float* xyz, float* out, uint32_t* steps);
 int launch_cast_rays(vct_context* c, int level, size_t n, const float* seg, uint32_t* voxel, float* t, uint8_t* face,
-                     uint8_t* rgba, uint32_t* steps);                                           // vct_view.cu, device pointers
+                     uint8_t* rgba, uint32_t* steps);                                           // vct_view.cu
 int check_overflow(vct_context* c);
 int comm_barrier(vct_context* c, int channel, cudaStream_t stream);   // device-side cross-rank barrier, in stream order
 int comm_check(vct_context* c);                                        // barrier time-outs -> VCT_ERR_STATE
@@ -264,6 +270,9 @@ int sync_all_streams(vct_context* c);      // main + voxel + visibility + copy s
 // launch shape of a grid-stride kernel of the voxel chain: `mult` blocks of 256 threads per SM
 #define VCT_CHAIN(mult) (unsigned)(148 * (mult)), 256u
 inline cudaError_t reset_item_queue(vct_context* c) { return cudaMemsetAsync(&c->d_counters->n_items, 0, 3 * sizeof(unsigned int), c->stream); }
+inline cudaError_t reset_steps(vct_context* c, StepCounter k) {
+  return cudaMemsetAsync(c->d_counters->steps[k], 0, sizeof(c->d_counters->steps[k]), c->stream);
+}
 
 // ------------------------------------------------------------------------------------ device helpers
 #ifdef __CUDACC__
@@ -278,6 +287,17 @@ __device__ __forceinline__ F4 mul_mat_vec(const float* __restrict__ m, float x, 
   r.z = ((m[2] * x + m[6] * y) + m[10] * z) + m[14] * w;
   r.w = ((m[3] * x + m[7] * y) + m[11] * z) + m[15] * w;
   return r;
+}
+
+// Adds the warp's sum of n to partial counter slot() (0..63) of step counter k: one atomic per warp, from lane 0.  The
+// kernel passes the lane it computed itself, and the slot as a callable evaluated only where the atomic is issued:
+// with threadIdx read in here, or the slot computed ahead of the reduction, nvcc 12.9 schedules the kernels and
+// allocates their registers differently.
+template <class Slot>
+__device__ __forceinline__ void count_steps(Counters* __restrict__ ctr, StepCounter k, unsigned lane, unsigned n, Slot slot) {
+#pragma unroll
+  for (int d = 16; d > 0; d >>= 1) n += __shfl_xor_sync(0xffffffffu, n, d);
+  if (lane == 0 && n) atomicAdd(&ctr->steps[k][slot() * 4], (unsigned long long)n);
 }
 
 // does this context render frame row j?  (row-band or interleaved-strip sharding of visibility and cone_trace)

@@ -141,14 +141,12 @@ __global__ void __launch_bounds__(256) voxel_view(Params P, Mat16 inv, int N, cu
     frame[(size_t)j * P.W + i] = out;
     if (voxel) voxel[(size_t)j * P.W + i] = idx;
   }
-#pragma unroll
-  for (int s = 16; s > 0; s >>= 1) steps += __shfl_xor_sync(0xffffffffu, steps, s);
-  if (lane == 0 && steps) atomicAdd(&ctr->view_steps[((blockIdx.x + blockIdx.y * 7u) & 63u) * 4], (unsigned long long)steps);
+  count_steps(ctr, STEPS_VIEW, lane, steps, [] { return (blockIdx.x + blockIdx.y * 7u) & 63u; });
 }
 
 int launch_voxel_view(vct_context* c, int level, const float inv_vp[16], uint32_t* d_voxel) {
   PassTimer timer(c, VCT_PASS_VOXEL_VIEW);
-  VCT_CUDA(c, cudaMemsetAsync(c->d_counters->view_steps, 0, sizeof(c->d_counters->view_steps), c->stream));
+  VCT_CUDA(c, reset_steps(c, STEPS_VIEW));
   Mat16 inv;
   for (int k = 0; k < 16; ++k) inv.m[k] = inv_vp[k];
   dim3 b(256), g((c->P.W + 31) / 32, (c->P.H + 7) / 8);
@@ -192,9 +190,7 @@ __global__ void __launch_bounds__(256) cast_rays_kernel(float G, int N, cudaSurf
     if (rgba) rgba[k] = c;
     if (steps_out) steps_out[k] = steps;
   }
-#pragma unroll
-  for (int s = 16; s > 0; s >>= 1) steps += __shfl_xor_sync(0xffffffffu, steps, s);
-  if ((threadIdx.x & 31) == 0 && steps) atomicAdd(&ctr->ray_steps[(blockIdx.x & 63u) * 4], (unsigned long long)steps);
+  count_steps(ctr, STEPS_RAYS, threadIdx.x & 31, steps, [] { return blockIdx.x & 63u; });
 }
 
 int launch_cast_rays(vct_context* c, int level, size_t n, const float* seg, uint32_t* voxel, float* t, uint8_t* face,
@@ -202,7 +198,7 @@ int launch_cast_rays(vct_context* c, int level, size_t n, const float* seg, uint
   const size_t blocks = (n + 255) / 256;
   if (blocks > 0x7fffffffu) return set_error(c, VCT_ERR_INVALID, "vct_cast_rays: too many segments for one launch");
   PassTimer timer(c, VCT_PASS_RAYS);
-  VCT_CUDA(c, cudaMemsetAsync(c->d_counters->ray_steps, 0, sizeof(c->d_counters->ray_steps), c->stream));
+  VCT_CUDA(c, reset_steps(c, STEPS_RAYS));
   cast_rays_kernel<<<(unsigned)blocks, 256, 0, c->stream>>>(c->P.grid_world, c->P.V >> level, c->grid[c->cur].surf[level],
                                                             c->grid_format == 1, n, seg, voxel, t, face, (uchar4*)rgba,
                                                             steps, c->d_counters);
